@@ -5,7 +5,7 @@ Workload (BASELINE.json configs[2], "C3"): RbQ10, MLP [2 -> 16 -> 16 -> 1] tanh,
 scale_nn_outputs, global Q10, mse, Adam(0.01), N = 2^24 synthetic Q10-shaped samples resident
 in HBM, batch 65536.  A "step" is one optimiser step on one batch.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 value      : samples/s, device-timed (CUDA events on the launching stream inside the library),
              data + index stream already resident in HBM.
@@ -16,6 +16,8 @@ roofline   : algorithmic bytes (16 B/sample) of one fused-step launch / its mean
 cpu_baseline: the oracle (CPU restatement of the reference algorithm; the reference itself is
              Julia and cannot run in this image) on all host cores, bounded sample.
 With --impl reference the same CPU implementation is what is timed.
+--dump-outputs DIR: after the K timed steps, DIR/<name>.npy holds what they hand their caller (see dump_outputs);
+             the inputs are seeded, so two builds run with the same arguments can be compared output for output.
 Multi-GPU (torchrun, one rank per GPU): weak scaling, every rank owns its own 2^24-sample shard
 and trains on per-GPU batches of 65536; gradients are combined once per step.
 """
@@ -31,6 +33,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (the tree may be read-only)
 
 B = 65536
 N_PER_GPU = 1 << 24
@@ -131,6 +134,15 @@ def wide_c5_leg(eh, device, rank=0, world=1, dist=None):
                          "peak_source": "MEASURED_PEAKS.json bf16_tflops_sustained" if peak else "unavailable",
                          "flops_counted": "hidden-layer GEMMs only (2 * 3 * 2 * B * 512 * 512 per step), per GPU"},
             "loss_first_last": [float(losses[0]), float(losses[-1])]}
+
+
+def dump_outputs(d, sess, losses):
+    """What the timed steps computed, as a caller of eh_run_steps receives it: the per-step losses of the timed call and,
+    after its last step, the trained parameters and the Adam moments (float32, a few KB in all)."""
+    os.makedirs(d, exist_ok=True)
+    m, v, _ = sess.get_opt_state()
+    for name, a in (("losses", losses), ("params", sess.get_params()), ("adam_m", m), ("adam_v", v)):
+        np.save(os.path.join(d, name + ".npy"), np.asarray(a, dtype=np.float32))
 
 
 def make_model(eh):
@@ -331,7 +343,10 @@ def main():
     ap.add_argument("--no-wide", action="store_true", help="skip the extra C5 (wide MLP, tcgen05) leg")
     ap.add_argument("--flags", type=int, default=0, help="EH_FLAG_* bits (1 = no CUDA graph, 2 = no PDL)")
     ap.add_argument("--no-e2e", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the timed steps to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         return run_reference(args)
 
@@ -388,6 +403,8 @@ def main():
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         dev_ms = float(t.item())
     value = world * K * B / (dev_ms * 1e-3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, sess, losses)
 
     # ---- roofline of the dominant kernel ----
     # The timed region is ONE launch of the persistent kernel k_epoch (all K steps, exchange included):

@@ -4,8 +4,6 @@ import ctypes
 import os
 import re
 
-import pytest
-
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -43,17 +41,26 @@ def test_struct_layout_matches_header(eh):
 
 
 def test_no_cpu_fallback(eh):
-    """without a CUDA device eh_create must fail with EH_ECUDA (and say so)"""
-    from conftest import rbq10_model
+    """without a CUDA device eh_create must fail with EH_ECUDA (and say so).  The session is created in a child process
+    that sees no device (CUDA_VISIBLE_DEVICES empty), so the check also runs on a machine that has a GPU."""
+    import subprocess
+    import sys
     from easyhybrid_b200 import _abi
-    try:
-        s = eh.FusedSession(rbq10_model(eh))
-    except eh.EasyHybridCudaError as e:
-        assert e.status == _abi.EH_ECUDA
-        assert "no CPU fallback" in str(e) or "sm_100a" in str(e)
-    else:
-        s.close()
-        pytest.skip("a CUDA device is present")
+    code = ("import sys; sys.path[:0] = [%r, %r]\n"
+            "import easyhybrid_b200 as eh\n"
+            "from conftest import rbq10_model\n"
+            "try:\n"
+            "    eh.FusedSession(rbq10_model(eh)).close()\n"
+            "except eh.EasyHybridCudaError as e:\n"
+            "    print(e.status)\n"
+            "    print(e)\n") % (ROOT, os.path.join(ROOT, "tests"))
+    r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=300,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
+    assert r.returncode == 0, r.stderr[-4000:]
+    out = r.stdout.split("\n", 1)
+    assert len(out) == 2, "eh_create succeeded without a visible CUDA device"
+    assert int(out[0]) == _abi.EH_ECUDA
+    assert "no CPU fallback" in out[1] or "sm_100a" in out[1]
 
 
 def test_product_does_not_import_oracle():

@@ -6,7 +6,7 @@ the per-step form eh_step_host on host batches) against include/easyhybrid_cuda.
 ctypes, no torch between the caller and the library.  The harness writes its inputs and results to files; this test
 checks the results against the CPU checker on exactly those inputs.
 
-CPU part: the harness compiles as C against the header, links against the library, and -- there being no GPU -- fails
+CPU part: the harness compiles as C against the header, links against the library, and -- with no GPU visible -- fails
 loudly instead of falling back."""
 import os
 import subprocess
@@ -29,10 +29,9 @@ def _build(tmp_path):
 
 def test_replay_harness_builds_as_c_and_fails_loudly_without_a_gpu(tmp_path):
     exe = _build(tmp_path)
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present: the gpu test runs the harness")
-    r = subprocess.run([exe, str(tmp_path / "out")], capture_output=True, text=True)
+    # the harness sees no device (CUDA_VISIBLE_DEVICES empty), also on a machine that has a GPU
+    r = subprocess.run([exe, str(tmp_path / "out")], capture_output=True, text=True,
+                       env=dict(os.environ, CUDA_VISIBLE_DEVICES=""))
     assert r.returncode == 3 and "no CPU fallback" in r.stderr, (r.returncode, r.stderr)
 
 
