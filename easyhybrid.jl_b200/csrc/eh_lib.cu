@@ -896,7 +896,8 @@ eh_status wide_run_steps(eh_ctx* c, int64_t n, int64_t B, int64_t first, int64_t
             for (int r = 0; r < c->world; r++) dp.peer[r] = reinterpret_cast<float*>(c->dp_peer[r]);
         }
         cudaError_t e = c->wide->step(sp.rec, c->d_idx + b * B, 0, (int)Bk, c->d_bscal + (size_t)b * BS_STRIDE, c->d_theta, c->d_m,
-                                      c->d_v, c->d_ost, c->d_grad, c->d_loss + k, apply, c->stream, c->world > 1 ? &dp : nullptr);
+                                      c->d_v, c->d_ost, c->d_grad, c->d_loss + k, apply, c->stream, c->world > 1 ? &dp : nullptr,
+                                      sp.shift_y);
         if (e != cudaSuccess) return fail(c, EH_ECUDA, "wide path: %s", c->wide->error());
         if (apply) CK(refresh_tail(c));
     }
@@ -912,7 +913,7 @@ eh_status wide_run_steps(eh_ctx* c, int64_t n, int64_t B, int64_t first, int64_t
         return fail(c, EH_ENCCL, "wide path: a data-parallel peer never published its gradient");
     }
     CK(cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1));
-    c->last_launches = nsteps * (3 + 5 * (int64_t)(c->var->NH - 1) + 4);
+    c->last_launches = nsteps * (3 + 5 * (int64_t)(c->var->NH - 1) + 4 + c->wide->extra_launches());
     c->last_step_ms = c->last_ms;
     if (losses) memcpy(losses, c->h_loss, (size_t)nsteps * sizeof(float));
     if (c->use_bn && apply) return update_bn_running(c, n, B, first, nsteps);
@@ -1253,7 +1254,7 @@ eh_status enqueue_host_step_compute(eh_ctx* c, HostStage& h, int64_t B, float* l
     if (c->wide) {
         if (c->world > 1) return fail(c, EH_EUNSUPPORTED, "host-batch steps of the tensor-core path are single-GPU: use eh_run_steps in data-parallel mode");
         cudaError_t we = c->wide->step(h.d_rec, nullptr, 0, (int)B, h.d_bscal, c->d_theta, c->d_m, c->d_v, c->d_ost, c->d_grad, loss_dst, 1,
-                                       c->stream, nullptr);
+                                       c->stream, nullptr, c->split[EH_SPLIT_TRAIN].shift_y);
         if (we != cudaSuccess) return fail(c, EH_ECUDA, "wide path: %s", c->wide->error());
         CK(refresh_tail(c));
         CK(cudaEventRecord(h.freed, c->stream));
@@ -1652,6 +1653,7 @@ eh_status eh_create(eh_ctx** out, const eh_model_desc* desc)
         CK(refresh_tail(c));
         if (v->engine == 3) {
             c->wide_model.d_slot_of_flat = c->d_slot_of_flat;
+            c->wide_model.d_l2coef = c->l2_on ? c->d_l2coef : nullptr;
             char werr[256] = {0};
             c->wide = eh::wide::WideNet::create(c->wide_model, werr, sizeof werr);
             if (!c->wide) return fail(c, EH_ECUDA, "%s", werr);
@@ -2170,6 +2172,10 @@ eh_status eh_comm_init(eh_ctx* c, int32_t rank, int32_t world, const void* ids)
         return fail(c, EH_EINVAL, "eh_comm_init: world must be 1..%d and 0 <= rank < world", EH_MAX_WORLD);
     if (!c->dp_block) return fail(c, EH_EINVAL, "eh_comm_init: call eh_comm_id on this ctx first");
     if (!c->persist_ok && !c->wide) return fail(c, EH_EUNSUPPORTED, "data-parallel mode needs the persistent kernel, unavailable for this model");
+    // (the seeds of these losses need statistics of the GLOBAL batch's predictions, which the ranks do not exchange)
+    if (c->wide && (c->stat_loss || c->l2_on))
+        return fail(c, EH_EUNSUPPORTED, "data-parallel mode on the tensor-core path: rmse over several targets, pearsonLoss, kgeLoss, "
+                                        "pbkgeLoss and weight_l2 train on one GPU only");
     EH_ENTER(c);
     for (int r = 0; r < world; r++) {
         if (r == rank) { c->dp_peer[r] = c->dp_block; continue; }

@@ -69,6 +69,8 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     memset(&wm, 0, sizeof wm);
     int off = 0, ioff = 0, ooff = 0, uoff[8] = {0};
     std::vector<int> out_row0((size_t)NC, 0);
+    std::vector<std::pair<int, int>> wranges;   // (flat offset, count) of every Dense weight matrix, with its chain in l2_chain
+    std::vector<int> l2_chain;
     auto push = [&](int kind, int l, int r, int cc) { c->h_wmap.push_back(kind); c->h_wmap.push_back(l); c->h_wmap.push_back(r); c->h_wmap.push_back(cc); };
     for (int k = 0; k < NC; k++) {
         const eh_chain_desc& ch = d->chains[k];
@@ -86,6 +88,8 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
             const int kind = l == 1 ? eh::wide::WK_W1 : (l <= NH ? eh::wide::WK_WH : eh::wide::WK_WO);
             for (int i = 0; i < hin; i++)
                 for (int o = 0; o < hout; o++) push(kind, l, ro + o, co + i);
+            wranges.push_back({off, hout * hin});
+            l2_chain.push_back(k);
             off += hout * hin;
             for (int o = 0; o < hout; o++) push(l <= NH ? eh::wide::WK_B : eh::wide::WK_BO, l, ro + o, 0);
             off += hout;
@@ -153,16 +157,31 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     }
     for (int t = 0; t < d->n_targ; t++) { c->src_kind[c->ncols] = 1; c->src_idx[c->ncols] = d->n_forc + t; c->ncols++; }
 
-    // loss / optimiser
-    int n_rmse = 0;
+    // loss / optimiser.  rmse over several targets and pearsonLoss / kgeLoss / pbkgeLoss need statistics of the batch's
+    // predictions before the seeds exist: those targets run as LOSS_AFFINE behind a statistics pass of the head kernel
+    // (WideNet::step); single-target rmse keeps LOSS_RMSE and its 1 / (2 rmse) factor
     for (int t = 0; t < d->n_targ; t++) {
         const int lk = d->loss_per_target[t];
         if (lk < 0 || lk > EH_LOSS_PBKGELOSS) return fail(c, EH_EINVAL, "loss_per_target[%d]=%d unknown", t, lk);
-        if (lk > EH_LOSS_NSELOSS) return fail(c, EH_EUNSUPPORTED, "pearsonLoss / kgeLoss / pbkgeLoss are not available on the tensor-core path (chains wider than 32)");
-        c->loss_kind[t] = lk;
-        if (lk == EH_LOSS_RMSE) n_rmse++;
+        c->loss_kind_abi[t] = lk;
+        const bool stat = lk >= EH_LOSS_PEARSONLOSS || (lk == EH_LOSS_RMSE && d->n_targ > 1);
+        c->loss_kind[t] = stat ? (int)LOSS_AFFINE : lk;
+        c->stat_loss |= stat;
     }
-    if (n_rmse && d->n_targ > 1) return fail(c, EH_EUNSUPPORTED, "rmse training loss with more than one target");
+    // native extra loss lambda * weight_l2(ps.<chains>; normalize) (ABI version 2), as on the exact-fp32 path: 2 lambda [/ n]
+    // on the Dense weight entries of the selected chains (every layer, output layer included), 0 elsewhere
+    c->l2_on = d->abi_version >= 2 && d->l2_lambda != 0.f;
+    if (c->l2_on) {
+        auto picked = [&](int k) { return !d->l2_chain_mask || ((d->l2_chain_mask >> k) & 1u); };
+        long long nw = 0;
+        for (size_t i = 0; i < wranges.size(); i++) nw += picked(l2_chain[i]) ? wranges[i].second : 0;
+        const double lam = (double)d->l2_lambda / ((d->l2_normalize && nw > 0) ? (double)nw : 1.0);
+        c->l2_aggw = d->agg == EH_AGG_MEAN ? 0.5f : 1.0f;
+        c->l2_loss_coef = (float)lam;
+        c->h_l2coef.assign((size_t)c->nflat, 0.f);
+        for (size_t i = 0; i < wranges.size(); i++)
+            for (int j = 0; picked(l2_chain[i]) && j < wranges[i].second; j++) c->h_l2coef[(size_t)wranges[i].first + j] = (float)(2.0 * lam);
+    }
     c->agg_mean = d->agg == EH_AGG_MEAN;
     c->opt_kind = d->opt_kind;
     if (c->opt_kind < 0 || c->opt_kind > 3) return fail(c, EH_EINVAL, "opt_kind=%d unknown", d->opt_kind);
@@ -175,7 +194,8 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     wm.h_map = c->h_wmap.data();
     wm.act = c0.activation; wm.scale = d->scale_nn_outputs ? 1 : 0; wm.pm = d->process_model;
     wm.T = v->T; wm.F = v->F; wm.NPS = v->NPS; wm.use_bn = c->use_bn; wm.agg_mean = c->agg_mean;
-    for (int t = 0; t < MAXT; t++) wm.loss_kind[t] = c->loss_kind[t];
+    for (int t = 0; t < MAXT; t++) { wm.loss_kind[t] = c->loss_kind[t]; wm.loss_kind_abi[t] = c->loss_kind_abi[t]; }
+    wm.l2_aggw = c->l2_aggw; wm.l2_loss_coef = c->l2_loss_coef;   // (d_l2coef: set when the device copy exists)
     for (int s2 = 0; s2 < MAXPS; s2++) {
         wm.slot[s2].role = c->slots[s2].role; wm.slot[s2].idx = c->slots[s2].idx; wm.slot[s2].lo = c->slots[s2].lo;
         wm.slot[s2].span = c->slots[s2].span; wm.slot[s2].fixedv = c->slots[s2].fixedv;
@@ -575,7 +595,6 @@ eh_status build_plan(eh_ctx* c, const eh_model_desc* d)
     // `weight` entries of the selected chains, 0 elsewhere
     c->l2_on = d->abi_version >= 2 && d->l2_lambda != 0.f;
     if (c->l2_on) {
-        if (wide) return fail(c, EH_EUNSUPPORTED, "weight_l2 extra loss is not available on the tensor-core path (chains wider than 32)");
         long long nw = 0;
         for (int k = 0; k < NC; k++)
             if (!d->l2_chain_mask || ((d->l2_chain_mask >> k) & 1u))

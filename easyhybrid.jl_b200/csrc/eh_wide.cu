@@ -6,6 +6,7 @@
 #include <vector>
 
 #include "../../include/easyhybrid_cuda.h"
+#include "eh_stat_seeds.cuh"
 #include "eh_wide.h"
 #include "eh_wide_gemm.cuh"
 #include "eh_wide_kernels.cuh"
@@ -174,19 +175,24 @@ cudaError_t gemm_wgrad(const CUtensorMap& tmD, const CUtensorMap& tmA, int M, in
 namespace {
 
 typedef void (*HeadKernel)(const HeadArgs);
-struct HeadEntry { int pm, nout, scale, hch; HeadKernel fn; };
-#define EH_HEAD(PMF, NOUT, SCALE, HCH) {PMF::ID, NOUT, SCALE, HCH, k_wide_head<HeadCfg<PMF, NOUT, (SCALE != 0)>, HCH>},
-#define EH_HEAD_PM(PMF) EH_HEAD(PMF, 1, 0, 1) EH_HEAD(PMF, 1, 1, 1) EH_HEAD(PMF, 2, 0, 1) EH_HEAD(PMF, 2, 1, 1) \
-                        EH_HEAD(PMF, 1, 0, 2) EH_HEAD(PMF, 1, 1, 2) EH_HEAD(PMF, 2, 0, 2) EH_HEAD(PMF, 2, 1, 2)
+struct HeadEntry { int pm, nout, scale, hch, aff; HeadKernel fn; };
+#define EH_HEAD(PMF, NOUT, SCALE, HCH, AFF) {PMF::ID, NOUT, SCALE, HCH, AFF, k_wide_head<HeadCfg<PMF, NOUT, (SCALE != 0), (AFF != 0)>, HCH>},
+#define EH_HEAD_PMA(PMF, AFF) EH_HEAD(PMF, 1, 0, 1, AFF) EH_HEAD(PMF, 1, 1, 1, AFF) EH_HEAD(PMF, 2, 0, 1, AFF) EH_HEAD(PMF, 2, 1, 1, AFF) \
+                              EH_HEAD(PMF, 1, 0, 2, AFF) EH_HEAD(PMF, 1, 1, 2, AFF) EH_HEAD(PMF, 2, 0, 2, AFF) EH_HEAD(PMF, 2, 1, 2, AFF)
+#define EH_HEAD_PM(PMF) EH_HEAD_PMA(PMF, 0) EH_HEAD_PMA(PMF, 1)
 const HeadEntry g_heads[] = {EH_HEAD_PM(PmRbQ10) EH_HEAD_PM(PmExpo) EH_HEAD_PM(PmLinear) EH_HEAD_PM(PmLinear2) EH_HEAD_PM(PmExpo2)
                              EH_HEAD_PM(PmProgram)};
 
-HeadKernel find_head(int pm, int nout, int scale, int hch)
+// aff: the training head of a model with LOSS_AFFINE targets (the statistics and evaluation modes take aff = 0)
+HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false)
 {
     for (const HeadEntry& e : g_heads)
-        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0) && e.hch == hch) return e.fn;
+        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0) && e.hch == hch && e.aff == (aff ? 1 : 0)) return e.fn;
     return nullptr;
 }
+
+// CTAs of k_wide_gradpost: a function of the shape only, so that its sums of theta^2 have one fixed order
+int gradpost_grid(const WideModel& m) { return std::max(1, std::min((m.nflat + 255) / 256, 2 * m.nsm)); }
 
 WideDims dims_of(const WideModel& m)
 {
@@ -225,11 +231,14 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
     };
     cudaError_t e = gemm_prepare();
     if (e != cudaSuccess) return bail("gemm_prepare", e);
-    HeadKernel hk = find_head(m.pm, m.NOUT, m.scale, m.H / 256);
-    if (!hk) { snprintf(err, errlen, "wide path: no head kernel for this process model / shape"); delete w; return nullptr; }
-    const int head_smem = (8 * (m.NOUT + 1) + m.NOUT) * m.H * (int)sizeof(float);   // warps' scratch / row rings + the output-layer weights
-    e = cudaFuncSetAttribute((const void*)hk, cudaFuncAttributeMaxDynamicSharedMemorySize, head_smem);
-    if (e != cudaSuccess) return bail("head smem", e);
+    for (int t = 0; t < m.T && t < 4; t++) w->affine_ |= m.loss_kind[t] == LOSS_AFFINE;
+    for (int aff = 0; aff <= (w->affine_ ? 1 : 0); aff++) {
+        HeadKernel hk = find_head(m.pm, m.NOUT, m.scale, m.H / 256, aff != 0);
+        if (!hk) { snprintf(err, errlen, "wide path: no head kernel for this process model / shape"); delete w; return nullptr; }
+        const int head_smem = (8 * (m.NOUT + 1) + m.NOUT) * m.H * (int)sizeof(float);   // warps' scratch / row rings + the output-layer weights
+        e = cudaFuncSetAttribute((const void*)hk, cudaFuncAttributeMaxDynamicSharedMemorySize, head_smem);
+        if (e != cudaSuccess) return bail("head smem", e);
+    }
     const size_t HH = (size_t)m.H * m.H;
     const int bn = w->persist_ ? pg_box_rows() : gemm_bn(GEMM_FWD);
     // images of the embedded chain: everything outside the real entries (padding, other chains' units) stays zero
@@ -288,6 +297,13 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
     if ((e = cudaMalloc(&w->skip_, 4)) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&w->evalpart_, (size_t)w->n_head_ * 4 * 8 * sizeof(double))) != cudaSuccess) return bail("cudaMalloc", e);
     cudaMemset(w->skip_, 0, 4);
+    for (int t = 0; t < m.T && t < 4; t++) w->post_ |= m.loss_kind[t] == LOSS_RMSE;
+    if (m.d_l2coef) {
+        w->post_ = true;
+        if ((e = cudaMalloc(&w->l2part_, (size_t)gradpost_grid(m) * 4)) != cudaSuccess) return bail("cudaMalloc", e);
+        if ((e = cudaMalloc(&w->ticket_, 4)) != cudaSuccess) return bail("cudaMalloc", e);
+        cudaMemset(w->ticket_, 0, 4);
+    }
     return w;
 }
 
@@ -303,7 +319,8 @@ WideNet::~WideNet()
         if (Bp_[i]) cudaFree(Bp_[i]);
         if (colsum_[i]) cudaFree(colsum_[i]);
     }
-    void* ps[] = {xb_, D_[0], D_[1], partial_, head_partial_, stats_, skip_, evalpart_, d_prog_, W1img_, WOimg_, BOimg_, d_map_, d_small_};
+    void* ps[] = {xb_, D_[0], D_[1], partial_, head_partial_, stats_, skip_, evalpart_, l2part_, ticket_, d_prog_, W1img_, WOimg_, BOimg_,
+                  d_map_, d_small_};
     for (void* p : ps)
         if (p) cudaFree(p);
 }
@@ -384,9 +401,9 @@ cudaError_t WideNet::forward(const float* rec, const int* idx, long long rec_bas
     return cudaSuccess;
 }
 
-cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, int Bvalid, const float* bscal, float* pblock,
+cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, int Bvalid, float* bscal, float* pblock,
                           float* m, float* v, void* ost, float* grad_final, float* loss_out, int apply, cudaStream_t st,
-                          const WideDp* dp)
+                          const WideDp* dp, const float* shift_y)
 {
     const int H = m_.H, NH = m_.NH;
     const int B = (Bvalid + 127) / 128 * 128;   // GEMM tiles are 128 rows: padded rows are masked in the head kernel
@@ -397,7 +414,7 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     WN(ensure(B));
     WN(forward(rec, idx, rec_base, 1ll << 62, B, Bvalid, bscal, pblock, st));
     const WideDims d = dims_of(m_);
-    HeadKernel hk = find_head(m_.pm, m_.NOUT, m_.scale, H / 256);
+    HeadKernel hk = find_head(m_.pm, m_.NOUT, m_.scale, H / 256, affine_);
     HeadArgs ha{};
     ha.A = A_[NH - 1]; ha.xb = xb_; ha.pblock = pblock; ha.WOimg = WOimg_; ha.BOimg = BOimg_; ha.bscal = bscal; ha.D = D_[NH & 1];
     ha.partial = head_partial_;
@@ -407,6 +424,23 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     for (int s = 0; s < 8; s++) { ha.slot[s].role = m_.slot[s].role; ha.slot[s].idx = m_.slot[s].idx; ha.slot[s].lo = m_.slot[s].lo; ha.slot[s].span = m_.slot[s].span; ha.slot[s].fixedv = m_.slot[s].fixedv; }
     for (int i = 0; i < 4; i++) ha.pmc[i] = m_.pmc[i];
     const int head_smem = (8 * (m_.NOUT + 1) + m_.NOUT) * H * (int)sizeof(float);
+    if (affine_) {
+        // prediction-statistics losses: the head kernel's statistics mode over the training forward (train-mode
+        // BatchNorm is in A_NH already) leaves per-CTA sufficient statistics of the batch; k_stat_seeds turns them into
+        // the seed coefficients and the loss value in the batch's scalar row, which the training head reads next
+        if (!shift_y) { snprintf(err_, sizeof err_, "step: prediction-statistics losses need the train split's shift_y"); return cudaErrorInvalidValue; }
+        HeadArgs hs = ha;
+        hs.train = 0; hs.D = nullptr; hs.partial = nullptr; hs.yhat = nullptr; hs.parout = nullptr; hs.ldy = 0; hs.row0 = 0;
+        hs.evalstat = evalpart_;
+        for (int t = 0; t < 4; t++) hs.shift_y[t] = shift_y[t];
+        find_head(m_.pm, m_.NOUT, m_.scale, H / 256)<<<n_head_, 256, head_smem, st>>>(hs);
+        WN(cudaGetLastError());
+        StatSeedArgs z{};
+        z.partial = evalpart_; z.nparts = n_head_; z.Tk = m_.T; z.T = m_.T; z.agg_mean = m_.agg_mean; z.bscal = bscal;
+        for (int t = 0; t < 4; t++) { z.kind[t] = m_.loss_kind[t] == LOSS_AFFINE ? m_.loss_kind_abi[t] : -1; z.shift_y[t] = shift_y[t]; }
+        k_stat_seeds<<<1, 32, 0, st>>>(z);
+        WN(cudaGetLastError());
+    }
     hk<<<n_head_, 256, head_smem, st>>>(ha);
     WN(cudaGetLastError());
     const bool fork = side_ != nullptr && !getenv("EH_WIDE_NO_SIDE_STREAM");
@@ -443,13 +477,23 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     fa.d = d; fa.head_partial = head_partial_; fa.n_head = n_head_; fa.n_slab = n_slab_;
     fa.map = reinterpret_cast<const ParamMap*>(d_map_); fa.small = d_small_; fa.n_small = n_small_;
     for (int l = 1; l < NH; l++) fa.colsum[l - 1] = colsum_[l - 1];
-    fa.bscal = bscal; fa.theta = pblock; fa.grad = grad; fa.stats = stats_; fa.loss_out = loss_out;
+    fa.bscal = bscal; fa.theta = pblock; fa.grad = grad; fa.stats = stats_; fa.loss_out = m_.d_l2coef ? nullptr : loss_out;
     fa.T = m_.T; fa.agg_mean = m_.agg_mean;
     for (int t = 0; t < 4; t++) fa.loss_kind[t] = m_.loss_kind[t];
     for (int s = 0; s < 8; s++) fa.slot[s] = ha.slot[s];
     fa.slot_of_flat = m_.d_slot_of_flat; fa.skip_out = skip_; fa.dp = isdp ? 1 : 0;
     k_wide_gradfin<<<(n_small_ + 31) / 32, 256, 0, st>>>(fa);
     WN(cudaGetLastError());
+    if (post_) {   // (single GPU only: data-parallel mode refuses rmse and weight_l2)
+        PostArgs pa{};
+        pa.map = reinterpret_cast<const ParamMap*>(d_map_); pa.nflat = m_.nflat; pa.theta = pblock; pa.grad = grad;
+        pa.stats = stats_; pa.bscal = bscal; pa.T = m_.T;
+        for (int t = 0; t < 4; t++) pa.loss_kind[t] = m_.loss_kind[t];
+        pa.l2coef = m_.d_l2coef; pa.l2_aggw = m_.l2_aggw; pa.l2_loss_coef = m_.l2_loss_coef;
+        pa.l2part = l2part_; pa.ticket = ticket_; pa.loss_out = loss_out;
+        k_wide_gradpost<<<gradpost_grid(m_), 256, 0, st>>>(pa);
+        WN(cudaGetLastError());
+    }
     if (isdp) {
         AllredArgs ar{};
         for (int r = 0; r < dp->world; r++) ar.peer[r] = dp->peer[r];
@@ -465,10 +509,8 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     if (apply) {
         WUpdArgs u{};
         u.d = d; u.theta = pblock; u.m = m; u.v = v; u.ost = reinterpret_cast<OptState*>(ost); u.grad = grad; u.skip = skip_;
-        u.stats = stats_; u.bscal = bscal; u.T = m_.T;
         u.map = reinterpret_cast<const ParamMap*>(d_map_);
         u.W1img = W1img_; u.WOimg = WOimg_; u.BOimg = BOimg_;
-        for (int t = 0; t < 4; t++) u.loss_kind[t] = m_.loss_kind[t];
         u.opt_kind = m_.opt_kind; u.adamw_coupled = m_.adamw_coupled;
         u.eta = m_.eta; u.beta1 = m_.beta1; u.beta2 = m_.beta2; u.eps = m_.eps; u.lambda = m_.lambda;
         for (int l = 1; l <= NH; l++) { u.Wf[l - 1] = Wf_[l - 1]; u.Wb[l - 1] = Wb_[l - 1]; u.Bp[l - 1] = Bp_[l - 1]; }

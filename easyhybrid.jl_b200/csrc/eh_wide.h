@@ -36,12 +36,17 @@ struct WideModel {          // filled by eh_lib's planner from the model descrip
     int n_blocks;                            // hidden weight blocks (one per chain and hidden layer l >= 2)
     struct { int l, flat_off, hout, hin, o_off, i_off; } blocks[32];
     int act, scale, pm, T, F, NPS, use_bn, agg_mean;
-    int loss_kind[4];
+    int loss_kind[4];                        // LOSS_AFFINE for the prediction-statistics losses (seeds from a statistics pass)
+    int loss_kind_abi[4];                    // the descriptor's loss kind per target (what k_stat_seeds evaluates)
     PSlotH slot[8];
     float pmc[4];
     int opt_kind, adamw_coupled;
     float eta, beta1, beta2, eps, lambda;
     const int* d_slot_of_flat;
+    // native extra loss lambda * weight_l2 (d_l2coef NULL: none): loss l2_aggw (L + l2_loss_coef sum theta^2 over the flagged
+    // entries), gradient l2_aggw (g + l2coef[p] theta[p])
+    const float* d_l2coef;
+    float l2_aggw, l2_loss_coef;
     int nsm;
     // traced process model (pm == PM_PROGRAM): eh_pm_instr fields, value ids of the targets
     int prog_len;
@@ -63,9 +68,15 @@ public:
     // bf16 weight images from the fp32 master parameters (after eh_set_params)
     cudaError_t refresh_images(float* pblock, float* m, float* v, void* ost, cudaStream_t st);
     // one optimiser step (apply = 1) or loss + gradient only (apply = 0) on `B` samples rec[idx[.]];
-    // grad: [nflat] device buffer receiving dL/dflat; loss_out: device (or pinned host) float
-    cudaError_t step(const float* rec, const int* idx, long long rec_base, int B, const float* bscal, float* pblock, float* m,
-                     float* v, void* ost, float* grad, float* loss_out, int apply, cudaStream_t st, const WideDp* dp = nullptr);
+    // grad: [nflat] device buffer receiving dL/dflat; loss_out: device (or pinned host) float.  bscal: the batch's scalar
+    // row (device); the statistics pass of the LOSS_AFFINE targets writes their seed coefficients into it.  shift_y: the
+    // train split's target shifts (read for LOSS_AFFINE targets only)
+    cudaError_t step(const float* rec, const int* idx, long long rec_base, int B, float* bscal, float* pblock, float* m,
+                     float* v, void* ost, float* grad, float* loss_out, int apply, cudaStream_t st, const WideDp* dp = nullptr,
+                     const float* shift_y = nullptr);
+    // launches step() adds to the base sequence: statistics pass + seeds (LOSS_AFFINE targets), gradient epilogue
+    // (single-target rmse, weight_l2)
+    int extra_launches() const { return (affine_ ? 2 : 0) + (post_ ? 1 : 0); }
     // bytes of the exchange block a rank exposes in data-parallel mode: [2][xlen] floats + flags
     size_t dp_block_bytes() const { return (size_t)2 * dp_xlen() * sizeof(float) + 256; }
     int dp_xlen() const { return (m_.nflat + 16 + 31) / 32 * 32; }
@@ -84,6 +95,8 @@ private:
     WideModel m_{};
     int cap_ = 0, mapB_ = 0, n_head_ = 0, n_slab_ = 0, ksplit_ = 1;
     bool persist_ = true;
+    bool affine_ = false;      // some target is LOSS_AFFINE: statistics pass of the head kernel + k_stat_seeds per step
+    bool post_ = false;        // single-target rmse or weight_l2: k_wide_gradpost finishes the flat gradient
     float* xb_ = nullptr;
     __nv_bfloat16* A_[8] = {nullptr};
     __nv_bfloat16* D_[2] = {nullptr, nullptr};
@@ -105,6 +118,8 @@ private:
     float* head_partial_ = nullptr;
     float* stats_ = nullptr;
     double* evalpart_ = nullptr;
+    float* l2part_ = nullptr;      // [gradpost CTAs] partial sums of theta^2 over the weight_l2 entries
+    unsigned* ticket_ = nullptr;   // CTAs of k_wide_gradpost that have finished (the last one writes the loss)
     int* skip_ = nullptr;
     CUtensorMap tmA_k_[8], tmA_mn_[8], tmD_k_[2], tmD_mn_[2], tmWf_[8], tmWb_[8];
     char err_[256] = {0};

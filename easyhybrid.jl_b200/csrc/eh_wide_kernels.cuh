@@ -10,7 +10,12 @@
 //   per hidden layer l = NH .. 2:   gemm_wgrad (dW_l partials), gemm_bwd (D_{l-1}; its epilogue also emits the column sums = db)
 //   k_wide_wreduce   split-K partials -> flat gradient (fixed order)
 //   k_wide_gradfin   remaining gradient entries (W_1, biases, output layer, phi) and the loss value
+//   k_wide_gradpost  (single-target rmse, weight_l2) rmse factor of the hidden weight blocks, weight_l2 term and its loss
 //   k_wide_update    optimiser over the flat vector, bf16 weight images for the next step
+// Prediction-statistics losses (rmse over several targets, pearsonLoss, kgeLoss, pbkgeLoss: LOSS_AFFINE targets) put two
+// launches between the forward GEMMs and the training head: k_wide_head in its statistics mode over A_NH (sufficient
+// statistics of the batch's predictions per CTA) and k_stat_seeds (eh_stat_seeds.cuh: seed coefficients and loss value
+// into the batch's scalar row).
 // Replaces Lux.Training.single_train_step! (src/training/epoch.jl:20-26) for wide chains; formulas: SURVEY 10.2-10.5.
 #pragma once
 #include <cuda_bf16.h>
@@ -118,12 +123,13 @@ __global__ void __launch_bounds__(256) k_wide_first(const float* __restrict__ xb
     }
 }
 
-// the pieces of StepCfg that resolve_params / the process-model functors look at
-template <class PM_, int NOUT_, bool SCALE_>
+// the pieces of StepCfg that resolve_params / the process-model functors look at.  AFF: the training mode knows LOSS_AFFINE
+// seeds (a separate instantiation: the kernel runs at its register limit, and the extra case must not cost the others)
+template <class PM_, int NOUT_, bool SCALE_, bool AFF_ = false>
 struct HeadCfg {
     using PM = PM_;
     static constexpr int NOUT = NOUT_, NPS = PM_::NPS, T = PM_::NT, F = PM_::NF;
-    static constexpr bool SCALE = SCALE_;
+    static constexpr bool SCALE = SCALE_, AFF = AFF_;
 };
 
 struct HeadArgs {
@@ -325,6 +331,10 @@ __global__ void __launch_bounds__(256, 3) k_wide_head(const HeadArgs a)
             if (a.loss_kind[t] == LOSS_MAE) {
                 lsum[t] += fabsf(rr);
                 gy[t] = rr > 0.f ? c : (rr < 0.f ? -c : 0.f);
+            } else if (HC::AFF && a.loss_kind[t] == LOSS_AFFINE) {
+                // dL/dyhat = sa + sb yhat + sc y (k_stat_seeds): the coefficients carry the aggregation weight, the loss value
+                // is in the scalar row already
+                gy[t] = m ? fmaf(a.bscal[BS_AFF + 2 * MAXT + t], y[t], fmaf(a.bscal[BS_AFF + MAXT + t], yh[t], a.bscal[BS_AFF + t])) : 0.f;
             } else {
                 lsum[t] = fmaf(rr, rr, lsum[t]);
                 gy[t] = 2.f * c * rr;
@@ -462,7 +472,7 @@ struct FinArgs {
     const float* bscal;
     const float* theta;
     float* grad;                                  // in/out flat gradient (hidden weight blocks already there)
-    float* stats;                                 // out [MAXT] loss sums
+    float* stats;                                 // out [MAXT] loss sums, [MAXT] the loss value (read by k_wide_gradpost)
     float* loss_out;                              // nullable
     int T, agg_mean;
     int loss_kind[MAXT];
@@ -508,7 +518,10 @@ __global__ void __launch_bounds__(256) k_wide_gradfin(const FinArgs a)
         const float n = a.bscal[BS_N + t], ss = a.bscal[BS_SS + t], acc = s_loss[t];
         ntot += n;
         if (a.loss_kind[t] == LOSS_RMSE) post = 1.f / (2.f * sqrtf(acc / n));
-        L += (a.loss_kind[t] == LOSS_NSELOSS) ? acc / ss : (a.loss_kind[t] == LOSS_RMSE ? sqrtf(acc / n) : acc / n);
+        L += (a.loss_kind[t] == LOSS_NSELOSS)  ? acc / ss
+             : (a.loss_kind[t] == LOSS_RMSE)   ? sqrtf(acc / n)
+             : (a.loss_kind[t] == LOSS_AFFINE) ? a.bscal[BS_AFF + 3 * MAXT + t]   // value left by k_stat_seeds
+                                               : acc / n;
     }
     if (a.agg_mean) L /= (float)a.T;
     if (a.dp) post = 1.f;   // rmse is refused in data-parallel mode
@@ -519,6 +532,7 @@ __global__ void __launch_bounds__(256) k_wide_gradfin(const FinArgs a)
             if (a.loss_out) *a.loss_out = ntot == 0.f ? __int_as_float(0x7fc00000) : L;
             *a.skip_out = ntot == 0.f;
             for (int t = 0; t < MAXT; t++) a.stats[t] = s_loss[t];
+            a.stats[MAXT] = L;
         }
     }
     const int q = blockIdx.x * 32 + (threadIdx.x >> 3), zl = threadIdx.x & 7;
@@ -571,6 +585,65 @@ __global__ void __launch_bounds__(256) k_wide_gradfin(const FinArgs a)
         }
         a.grad[p] = s * post;
     }
+}
+
+struct PostArgs {
+    const ParamMap* map; int nflat;
+    const float* theta;                           // parameters before this step's update
+    float* grad;                                  // in/out flat gradient (complete after k_wide_gradfin)
+    const float* stats;                           // [MAXT] loss sums, [MAXT] loss value (k_wide_gradfin)
+    const float* bscal;
+    int T;
+    int loss_kind[MAXT];
+    const float* l2coef;                          // nullable [nflat]: 2 l2_loss_coef on the weight_l2 entries, else 0
+    float l2_aggw, l2_loss_coef;
+    float* l2part;                                // [gridDim.x] CTA sums of theta^2 over the weight_l2 entries
+    unsigned* ticket;                             // CTAs done (zero between launches)
+    float* loss_out;                              // nullable
+};
+
+// ---- the last pass over the flat gradient, for the loss terms that need all of it (exact path: k_update) ----
+// single-target rmse: the hidden weight blocks come straight from the GEMM partials, without the 1 / (2 rmse) that
+// k_wide_gradfin applies to every other entry.  weight_l2: g <- l2_aggw (g + l2coef[p] theta[p]) for every entry, and the
+// loss l2_aggw (L + l2_loss_coef sum theta^2) -- the sum over the flagged entries in a fixed order: per CTA (thread stride,
+// warp tree, warps in order), then the CTA sums in order by the CTA that finishes last.
+__global__ void __launch_bounds__(256) k_wide_gradpost(const PostArgs a)
+{
+    float post = 1.f;
+    for (int t = 0; t < a.T; t++)
+        if (a.loss_kind[t] == LOSS_RMSE) post = 1.f / (2.f * sqrtf(a.stats[t] / a.bscal[BS_N + t]));
+    float s = 0.f;
+    for (int p = blockIdx.x * blockDim.x + threadIdx.x; p < a.nflat; p += gridDim.x * blockDim.x) {
+        float g = a.grad[p];
+        if (post != 1.f && a.map[p].kind == WK_WH) g *= post;
+        if (a.l2coef) {
+            const float th = a.theta[p], c = a.l2coef[p];
+            if (c != 0.f) s = fmaf(th, th, s);
+            g = a.l2_aggw * fmaf(c, th, g);
+        }
+        a.grad[p] = g;
+    }
+    if (!a.l2coef) return;
+    __shared__ float s_w[8];
+    __shared__ bool s_last;
+    s = warp_sum(s);
+    if ((threadIdx.x & 31) == 0) s_w[threadIdx.x >> 5] = s;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        float cta = 0.f;
+        for (int w = 0; w < (int)(blockDim.x >> 5); w++) cta += s_w[w];
+        a.l2part[blockIdx.x] = cta;
+        __threadfence();   // the CTA sum is visible before the ticket says so
+        s_last = atomicAdd(a.ticket, 1u) == gridDim.x - 1;
+    }
+    __syncthreads();
+    if (!s_last || threadIdx.x != 0) return;
+    __threadfence();
+    float S = 0.f, ntot = 0.f;
+    for (int g = 0; g < (int)gridDim.x; g++) S += __ldcg(a.l2part + g);
+    for (int t = 0; t < a.T; t++) ntot += a.bscal[BS_N + t];
+    if (a.loss_out) *a.loss_out = ntot == 0.f ? __int_as_float(0x7fc00000) : a.l2_aggw * (a.stats[MAXT] + a.l2_loss_coef * S);
+    *a.ticket = 0u;
 }
 
 // ---- data parallel (one process per GPU): gradient all-reduce over NVLink peer memory ----
@@ -643,9 +716,6 @@ struct WUpdArgs {
     float* theta; float* m; float* v; OptState* ost;
     const float* grad;
     const int* skip;
-    const float* stats;        // loss sums (for the rmse post factor of the hidden blocks)
-    const float* bscal;
-    int loss_kind[MAXT]; int T;
     int opt_kind, adamw_coupled;
     float eta, beta1, beta2, eps, lambda;
     // images of the embedded chain, all zero outside the real entries
@@ -666,11 +736,7 @@ __global__ void __launch_bounds__(256) k_wide_update(const WUpdArgs a)
     const ParamMap mp = a.map[p];
     float th = a.theta[p];
     if (a.apply && !*a.skip) {
-        float g = a.grad[p];
-        // hidden weight blocks come straight from the GEMM partials: apply the rmse factor here
-        if (mp.kind == WK_WH)
-            for (int t = 0; t < a.T; t++)
-                if (a.loss_kind[t] == LOSS_RMSE) g *= 1.f / (2.f * sqrtf(a.stats[t] / a.bscal[BS_N + t]));
+        const float g = a.grad[p];
         const float b1t = a.ost->b1t, b2t = a.ost->b2t;
         float dx;
         if (a.opt_kind == OPT_ADAM || a.opt_kind == OPT_ADAMW) {

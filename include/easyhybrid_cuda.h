@@ -78,9 +78,9 @@ typedef enum { EH_ROLE_NEURAL = 0, EH_ROLE_GLOBAL = 1, EH_ROLE_FIXED = 2 } eh_ro
 
 /* per-target loss (src/losses/loss_fn.jl:58-81) */
 /* training losses of src/losses/loss_fn.jl:58-179.  The last three (and rmse over more than one target) depend on
- * statistics of the batch's PREDICTIONS (mean, variance, covariance with the observations): their steps run a forward
- * pre-pass over the batch first and take the one-launch-pair-per-step path (no persistent kernel, single GPU, exact-fp32
- * kernels only).                                                                                                      */
+ * statistics of the batch's PREDICTIONS (mean, variance, covariance with the observations): on the exact-fp32 kernels
+ * their steps run a forward pre-pass over the batch first and take the one-launch-pair-per-step path (no persistent
+ * kernel), on the tensor-core path (chains wider than 32) a statistics pass of the head kernel; single GPU on both.   */
 typedef enum {
     EH_LOSS_MSE = 0, EH_LOSS_RMSE = 1, EH_LOSS_MAE = 2, EH_LOSS_NSELOSS = 3,
     EH_LOSS_PEARSONLOSS = 4, /* 1 - cor(yhat, y)                                                loss_fn.jl:75-77   */

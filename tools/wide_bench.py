@@ -1,4 +1,9 @@
-"""C5 workload driver: multi-target Expo hybrid, hidden 3x512, PerTarget(nseLoss, mse), batch 65536 (SURVEY 8d)."""
+"""C5 workload driver: multi-target Expo hybrid, hidden 3x512, PerTarget(nseLoss, mse), batch 65536 (SURVEY 8d).
+
+usage: wide_bench.py [STEPS] [--loss nseLoss,mse] [--weight-l2 LAMBDA]
+--loss: one training loss per target (comma separated), e.g. kgeLoss,mse; --weight-l2: add the extra loss
+LAMBDA * weight_l2(ps).  Without them the workload is the C5 one and the printed line is unchanged."""
+import argparse
 import os
 import sys
 import time
@@ -28,8 +33,19 @@ def make_model():
 
 
 def main():
+    ap = argparse.ArgumentParser(description="C5 step time on the tensor-core path")
+    ap.add_argument("steps", nargs="?", type=int, default=32)
+    ap.add_argument("--loss", default="nseLoss,mse", help="training loss per target, comma separated")
+    ap.add_argument("--weight-l2", type=float, default=0.0, metavar="LAMBDA", help="extra loss LAMBDA * weight_l2(ps)")
+    args = ap.parse_args()
     log2n = int(os.environ.get("EH_WIDE_LOG2N", "20"))
-    steps = int(sys.argv[1]) if len(sys.argv) > 1 else 32
+    steps = args.steps
+    losses_per_target = [x.strip() for x in args.loss.split(",")]
+    if len(losses_per_target) not in (1, 2):
+        ap.error("--loss: one loss for both targets or one per target")
+    training_loss = losses_per_target[0] if len(losses_per_target) == 1 else eh.PerTarget(*losses_per_target)
+    extra = eh.WeightL2(args.weight_l2) if args.weight_l2 else None
+    default = args.loss == "nseLoss,mse" and not args.weight_l2
     rank, world = int(os.environ.get("RANK", "0")), int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
     dist = None
@@ -41,7 +57,7 @@ def main():
     n = 1 << log2n
     model = make_model()
     xf, y = eh.prepare_data(model, synth(n, 2314 + rank))
-    sess = eh.FusedSession(model, training_loss=eh.PerTarget("nseLoss", "mse"), agg="sum", opt=eh.Adam(0.001), device=local)
+    sess = eh.FusedSession(model, training_loss=training_loss, agg="sum", opt=eh.Adam(0.001), device=local, extra_loss=extra)
     sess.upload(0, xf, y)
     sess.set_params(model.initialparameters(np.random.default_rng(0)))
     if world > 1:
@@ -66,7 +82,8 @@ def main():
     if rank == 0:
         print(f"wide C5 x{world}: {steps} steps, {1e3 * ms / steps:.1f} us/step (device, max over ranks), "
               f"{world * B * steps / (ms * 1e-3):.3e} samples/s, {flop * steps / (ms * 1e-3) / 1e12:.1f} TFLOP/s in the hidden GEMMs, "
-              f"wall {1e3 * (t1 - t0):.1f} ms, loss {losses[0]:.4f} -> {losses[-1]:.4f}")
+              f"wall {1e3 * (t1 - t0):.1f} ms, loss {losses[0]:.4f} -> {losses[-1]:.4f}"
+              + ("" if default else f" [loss {args.loss}" + (f", weight_l2 {args.weight_l2:g}" if args.weight_l2 else "") + "]"))
     sess.close()
     if dist is not None:
         dist.destroy_process_group()
