@@ -913,7 +913,7 @@ eh_status wide_run_steps(eh_ctx* c, int64_t n, int64_t B, int64_t first, int64_t
         return fail(c, EH_ENCCL, "wide path: a data-parallel peer never published its gradient");
     }
     CK(cudaEventElapsedTime(&c->last_ms, c->ev0, c->ev1));
-    c->last_launches = nsteps * (3 + 5 * (int64_t)(c->var->NH - 1) + 4 + c->wide->extra_launches());
+    c->last_launches = nsteps * (c->wide->base_launches() + 1 + c->wide->extra_launches());   // (+1: refresh_tail)
     c->last_step_ms = c->last_ms;
     if (losses) memcpy(losses, c->h_loss, (size_t)nsteps * sizeof(float));
     if (c->use_bn && apply) return update_bn_running(c, n, B, first, nsteps);

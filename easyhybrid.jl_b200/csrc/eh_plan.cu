@@ -35,11 +35,13 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     if (NH > 7 || !eh::wide::WideNet::supported(P, hmax, NH, NOUT, c0.activation, d->process_model))
         return fail(c, EH_EUNSUPPORTED,
                     "no fused kernel for this model: the register-tile kernels serve 1..3 hidden layers of summed width <= 32 "
-                    "(all activations, <= 8 inputs, <= 2 outputs); the tensor-core path serves 1..4 chains of equal "
-                    "depth (2..6 hidden layers, summed width per layer <= 512, <= 8 inputs and <= 2 outputs in total, tanh / sigmoid "
-                    "/ relu) (got process_model=%d chains=%d inputs=%d hidden=%d x (<= %d) outputs=%d activation=%d)",
+                    "(all activations, <= 8 inputs, <= 2 outputs); the wide path serves 1..4 chains of equal depth, activation "
+                    "and input_batchnorm with <= 8 inputs and <= 2 outputs in total: one hidden layer of summed width 33..512 "
+                    "(exact fp32, all activations) or 2..6 hidden layers of summed width <= 512 per layer (bf16 tensor cores, "
+                    "tanh / sigmoid / relu) (got process_model=%d chains=%d inputs=%d hidden=%d x (<= %d) outputs=%d activation=%d)",
                     d->process_model, NC, P, NH, hmax, NOUT, c0.activation);
-    const int HP = eh::wide::WideNet::padded_width(hmax);
+    // (one hidden layer: the fused exact-fp32 kernel k_wide_one, images padded to a multiple of 64 units)
+    const int HP = NH == 1 ? eh::wide::WideNet::one_width(hmax) : eh::wide::WideNet::padded_width(hmax);
     Variant& wv = c->wide_var;
     memset(&wv, 0, sizeof wv);
     wv.pm = d->process_model; wv.P = P; wv.NH = NH; wv.H = HP; wv.NOUT = NOUT; wv.act = c0.activation;
@@ -49,7 +51,7 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     wv.T = is_prog ? d->n_targ : ((d->process_model == EH_PM_LINEAR2 || d->process_model == EH_PM_EXPO2) ? 2 : 1);
     wv.R4 = rup4(wv.P + wv.F + wv.T);
     wv.NW = 0; wv.NPART = NSTAT; wv.off_stats = 0; wv.stage_floats = NSTAT; wv.max_warps = 8;
-    wv.name = "wide/bf16-tcgen05";
+    wv.name = NH == 1 ? "wide/fp32-one-hidden" : "wide/bf16-tcgen05";
     if (wv.T != d->n_targ) return fail(c, EH_EINVAL, "process model yields %d targets, descriptor has %d", wv.T, d->n_targ);
     const Variant* v = &wv;
     c->var = v; c->var2 = nullptr;

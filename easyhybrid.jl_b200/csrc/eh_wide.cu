@@ -10,6 +10,7 @@
 #include "eh_wide.h"
 #include "eh_wide_gemm.cuh"
 #include "eh_wide_kernels.cuh"
+#include "eh_wide_one.cuh"
 
 namespace eh {
 namespace wide {
@@ -191,6 +192,21 @@ HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false)
     return nullptr;
 }
 
+// the fused kernel of one hidden layer: one instantiation per process model, output count and scale_nn_outputs
+// (activation, input count, mode and loss kinds are run-time arguments)
+typedef void (*OneKernel)(const OneArgs);
+struct OneEntry { int pm, nout, scale; OneKernel fn; };
+#define EH_ONE(PMF, NOUT, SCALE) {PMF::ID, NOUT, SCALE, k_wide_one<HeadCfg<PMF, NOUT, (SCALE != 0)>>},
+#define EH_ONE_PM(PMF) EH_ONE(PMF, 1, 0) EH_ONE(PMF, 1, 1) EH_ONE(PMF, 2, 0) EH_ONE(PMF, 2, 1)
+const OneEntry g_ones[] = {EH_ONE_PM(PmRbQ10) EH_ONE_PM(PmExpo) EH_ONE_PM(PmLinear) EH_ONE_PM(PmLinear2) EH_ONE_PM(PmExpo2)
+                           EH_ONE_PM(PmProgram)};
+OneKernel find_one(int pm, int nout, int scale)
+{
+    for (const OneEntry& e : g_ones)
+        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0)) return e.fn;
+    return nullptr;
+}
+
 // CTAs of k_wide_gradpost: a function of the shape only, so that its sums of theta^2 have one fixed order
 int gradpost_grid(const WideModel& m) { return std::max(1, std::min((m.nflat + 255) / 256, 2 * m.nsm)); }
 
@@ -213,6 +229,11 @@ WideDims dims_of(const WideModel& m)
 
 bool WideNet::supported(int P, int hmax, int NH, int NOUT, int act, int pm)
 {
+    if (NH == 1) {   // (one layer of <= 32 units belongs to the register-tile kernels)
+        if (P < 1 || P > WIDE_MAXP || NOUT < 1 || NOUT > 2 || hmax <= 32 || hmax > 512) return false;
+        if (act != ACT_TANH && act != ACT_SIGMOID && act != ACT_RELU && act != ACT_IDENTITY && act != ACT_SWISH) return false;
+        return find_one(pm, NOUT, 0) != nullptr;
+    }
     if (P < 1 || P > WIDE_MAXP || NH < 2 || NH > 6 || NOUT < 1 || NOUT > 2) return false;
     if (hmax < 1 || hmax > 512) return false;
     if (act != ACT_TANH && act != ACT_SIGMOID && act != ACT_RELU && act != ACT_IDENTITY) return false;
@@ -229,10 +250,26 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
         delete w;
         return nullptr;
     };
-    cudaError_t e = gemm_prepare();
-    if (e != cudaSuccess) return bail("gemm_prepare", e);
+    cudaError_t e = cudaSuccess;
     for (int t = 0; t < m.T && t < 4; t++) w->affine_ |= m.loss_kind[t] == LOSS_AFFINE;
-    for (int aff = 0; aff <= (w->affine_ ? 1 : 0); aff++) {
+    if (m.NH == 1) {
+        // one hidden layer: no GEMM images, tensor maps, activation buffers or head kernel; k_wide_one's partial buffers
+        // have one row per CTA it can keep resident
+        OneKernel ok = find_one(m.pm, m.NOUT, m.scale);
+        if (!ok || m.H % 64 || m.H > 512 || m.R4 > WIDE_MAXP + ONE_FY) {
+            snprintf(err, errlen, "wide path: no fused one-hidden-layer kernel for this process model / shape");
+            delete w;
+            return nullptr;
+        }
+        w->one_fn_ = (void*)ok;
+        int per_sm = 0;
+        e = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, ok, one_block(m.H), one_smem(m.H, m.P, m.NOUT));
+        if (e != cudaSuccess) return bail("occupancy", e);
+        w->one_max_ = std::max(1, per_sm) * m.nsm;
+    } else if ((e = gemm_prepare()) != cudaSuccess) {
+        return bail("gemm_prepare", e);
+    }
+    for (int aff = 0; aff <= (w->affine_ ? 1 : 0) && m.NH >= 2; aff++) {
         HeadKernel hk = find_head(m.pm, m.NOUT, m.scale, m.H / 256, aff != 0);
         if (!hk) { snprintf(err, errlen, "wide path: no head kernel for this process model / shape"); delete w; return nullptr; }
         const int head_smem = (8 * (m.NOUT + 1) + m.NOUT) * m.H * (int)sizeof(float);   // warps' scratch / row rings + the output-layer weights
@@ -256,6 +293,10 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
             delete w;
             return nullptr;
         }
+    }
+    if (m.NH == 1) {
+        const size_t cs = (size_t)w->one_max_ * (1 + m.P) * m.H * 4;
+        if ((e = cudaMalloc(&w->colsum_[0], cs)) != cudaSuccess) return bail("cudaMalloc", e);
     }
     if ((e = cudaMalloc(&w->W1img_, (size_t)WIDE_MAXP * m.H * 4)) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&w->WOimg_, (size_t)4 * m.H * 4)) != cudaSuccess) return bail("cudaMalloc", e);
@@ -285,7 +326,7 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
         if ((e = cudaMalloc(&w->d_prog_, sizeof pd)) != cudaSuccess) return bail("cudaMalloc", e);
         if ((e = cudaMemcpy(w->d_prog_, &pd, sizeof pd, cudaMemcpyHostToDevice)) != cudaSuccess) return bail("cudaMemcpy", e);
     }
-    w->n_head_ = 3 * m.nsm;   // three CTAs of the head kernel are resident per SM (80 registers)
+    w->n_head_ = m.NH == 1 ? w->one_max_ : 3 * m.nsm;   // three CTAs of the head kernel are resident per SM (80 registers)
     if (cudaStreamCreateWithFlags(&w->side_, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&w->ev_wgrad_, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&w->ev_wred_, cudaEventDisableTiming) != cudaSuccess) {
         cudaGetLastError();
@@ -411,6 +452,21 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     const int par = isdp ? (int)(dp->tag & 1u) : 0;
     // data parallel: this rank's gradient goes into its exchange block, the all-reduce leaves the sum in grad_final
     float* grad = isdp ? dp->peer[dp->rank] + (size_t)par * dp_xlen() : grad_final;
+    if (NH == 1) {
+        // prediction-statistics losses: k_wide_one's statistics mode (forward only) then k_stat_seeds, as below
+        int g1 = 0;
+        if (affine_) {
+            if (!shift_y) { snprintf(err_, sizeof err_, "step: prediction-statistics losses need the train split's shift_y"); return cudaErrorInvalidValue; }
+            WN(launch_one(ONE_STATS, rec, idx, rec_base, 1ll << 62, Bvalid, bscal, pblock, nullptr, nullptr, 0, 0, evalpart_, shift_y, st, &g1));
+            StatSeedArgs z{};
+            z.partial = evalpart_; z.nparts = g1; z.Tk = m_.T; z.T = m_.T; z.agg_mean = m_.agg_mean; z.bscal = bscal;
+            for (int t = 0; t < 4; t++) { z.kind[t] = m_.loss_kind[t] == LOSS_AFFINE ? m_.loss_kind_abi[t] : -1; z.shift_y[t] = shift_y[t]; }
+            k_stat_seeds<<<1, 32, 0, st>>>(z);
+            WN(cudaGetLastError());
+        }
+        WN(launch_one(ONE_TRAIN, rec, idx, rec_base, 1ll << 62, Bvalid, bscal, pblock, nullptr, nullptr, 0, 0, nullptr, shift_y, st, &g1));
+        return finish_step(g1, g1, bscal, pblock, m, v, ost, grad, grad_final, loss_out, apply, st, dp);
+    }
     WN(ensure(B));
     WN(forward(rec, idx, rec_base, 1ll << 62, B, Bvalid, bscal, pblock, st));
     const WideDims d = dims_of(m_);
@@ -473,14 +529,27 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
                         (l - 1 == 1) ? m_.P : 0, m_.use_bn));
     }
     if (pending) WN(cudaStreamWaitEvent(st, ev_wred_, 0));   // the flat gradient is complete from here on
+    return finish_step(n_head_, n_slab_, bscal, pblock, m, v, ost, grad, grad_final, loss_out, apply, st, dp);
+}
+
+// the step's tail after the partials exist: gradient entries outside the hidden weight blocks and the loss (k_wide_gradfin),
+// the gradient epilogue, the data-parallel all-reduce, the optimiser
+cudaError_t WideNet::finish_step(int n_head, int n_slab, const float* bscal, float* pblock, float* m, float* v, void* ost,
+                                 float* grad, float* grad_final, float* loss_out, int apply, cudaStream_t st, const WideDp* dp)
+{
+    const int NH = m_.NH;
+    const bool isdp = dp && dp->world > 1;
+    const int par = isdp ? (int)(dp->tag & 1u) : 0;
+    const WideDims d = dims_of(m_);
     FinArgs fa{};
-    fa.d = d; fa.head_partial = head_partial_; fa.n_head = n_head_; fa.n_slab = n_slab_;
+    fa.d = d; fa.head_partial = head_partial_; fa.n_head = n_head; fa.n_slab = n_slab;
     fa.map = reinterpret_cast<const ParamMap*>(d_map_); fa.small = d_small_; fa.n_small = n_small_;
     for (int l = 1; l < NH; l++) fa.colsum[l - 1] = colsum_[l - 1];
+    if (NH == 1) fa.colsum[0] = colsum_[0];   // (one hidden layer: the W1 sums k_wide_one leaves, one slab per CTA)
     fa.bscal = bscal; fa.theta = pblock; fa.grad = grad; fa.stats = stats_; fa.loss_out = m_.d_l2coef ? nullptr : loss_out;
     fa.T = m_.T; fa.agg_mean = m_.agg_mean;
     for (int t = 0; t < 4; t++) fa.loss_kind[t] = m_.loss_kind[t];
-    for (int s = 0; s < 8; s++) fa.slot[s] = ha.slot[s];
+    for (int s = 0; s < 8; s++) { fa.slot[s].role = m_.slot[s].role; fa.slot[s].idx = m_.slot[s].idx; fa.slot[s].lo = m_.slot[s].lo; fa.slot[s].span = m_.slot[s].span; fa.slot[s].fixedv = m_.slot[s].fixedv; }
     fa.slot_of_flat = m_.d_slot_of_flat; fa.skip_out = skip_; fa.dp = isdp ? 1 : 0;
     k_wide_gradfin<<<(n_small_ + 31) / 32, 256, 0, st>>>(fa);
     WN(cudaGetLastError());
@@ -523,6 +592,34 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     return cudaSuccess;
 }
 
+// CTAs of k_wide_one for B rows: a function of the shape and B only (fixed tiles per CTA: a reproducible step)
+int WideNet::one_grid(int B) const
+{
+    const int tiles = (B + one_tile_rows(m_.H) - 1) / one_tile_rows(m_.H);
+    return std::max(1, std::min(tiles, one_max_));
+}
+
+cudaError_t WideNet::launch_one(int mode, const float* rec, const int* idx, long long rec_base, long long nrec, int B, const float* bscal,
+                                const float* pblock, float* yhat, float* parout, long long ldy, long long row0, double* evalstat,
+                                const float* shift_y, cudaStream_t st, int* grid_out)
+{
+    OneArgs a{};
+    a.rec = rec; a.idx = idx; a.rec_base = rec_base; a.nrec = nrec;
+    a.pblock = pblock; a.W1img = W1img_; a.b1img = Bp_[0]; a.WOimg = WOimg_; a.BOimg = BOimg_; a.bscal = bscal;
+    a.partial = head_partial_; a.colsum = colsum_[0];
+    a.yhat = yhat; a.parout = parout; a.ldy = ldy; a.row0 = row0; a.evalstat = evalstat;
+    for (int t = 0; t < 4; t++) { a.shift_y[t] = shift_y ? shift_y[t] : 0.f; a.loss_kind[t] = m_.loss_kind[t]; }
+    a.d = dims_of(m_); a.B = B; a.act = m_.act; a.mode = mode; a.use_bn = m_.use_bn;
+    for (int s = 0; s < 8; s++) { a.slot[s].role = m_.slot[s].role; a.slot[s].idx = m_.slot[s].idx; a.slot[s].lo = m_.slot[s].lo; a.slot[s].span = m_.slot[s].span; a.slot[s].fixedv = m_.slot[s].fixedv; }
+    for (int i = 0; i < 4; i++) a.pmc[i] = m_.pmc[i];
+    a.prog = reinterpret_cast<const PmProgData*>(d_prog_); a.nf = m_.F; a.nt = m_.T;
+    const int grid = one_grid(B);
+    reinterpret_cast<OneKernel>(one_fn_)<<<grid, one_block(m_.H), one_smem(m_.H, m_.P, m_.NOUT), st>>>(a);
+    WN(cudaGetLastError());
+    *grid_out = grid;
+    return cudaSuccess;
+}
+
 __global__ void k_wide_evalsum(const double* part, int n, int cnt, double* acc)
 {
     const int q = threadIdx.x;
@@ -537,6 +634,16 @@ cudaError_t WideNet::eval_rows(const float* rec, long long nrec, long long row0,
                                cudaStream_t st)
 {
     const int H = m_.H, NH = m_.NH;
+    if (NH == 1) {
+        int g1 = 0;
+        WN(launch_one(ONE_EVAL, rec, nullptr, row0, nrec, Bvalid, bscal, pblock, yhat, parout, ldy, row0, evalstat_dev ? evalpart_ : nullptr,
+                      shift_y, st, &g1));
+        if (evalstat_dev) {
+            k_wide_evalsum<<<1, 64, 0, st>>>(evalpart_, g1, m_.T * 8, evalstat_dev);
+            WN(cudaGetLastError());
+        }
+        return cudaSuccess;
+    }
     const int B = (Bvalid + 127) / 128 * 128;
     WN(ensure(B));
     WN(forward(rec, nullptr, row0, nrec, B, B, bscal, pblock, st));

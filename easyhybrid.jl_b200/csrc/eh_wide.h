@@ -58,9 +58,12 @@ struct WideModel {          // filled by eh_lib's planner from the model descrip
 // the wide-chain training step: owns activations / deltas / bf16 weight images / partial buffers
 class WideNet {
 public:
-    // hmax: widest embedded hidden layer (padded up to 256 or 512 inside)
+    // hmax: widest embedded hidden layer (padded up to 256 or 512 inside; one hidden layer: to a multiple of 64)
     static bool supported(int P, int hmax, int NH, int NOUT, int act, int pm);
     static int padded_width(int hmax) { return hmax <= 256 ? 256 : 512; }
+    // one hidden layer of 33..512 units (any activation, swish included) trains in the fused exact-fp32 kernel k_wide_one
+    // (eh_wide_one.cuh); its images are padded to a multiple of 64 units
+    static int one_width(int hmax) { return (hmax + 63) / 64 * 64; }
     static WideNet* create(const WideModel& m, char* err, size_t errlen);
     ~WideNet();
     // any batch size: rows are padded up to a multiple of 128 inside and masked
@@ -77,6 +80,9 @@ public:
     // launches step() adds to the base sequence: statistics pass + seeds (LOSS_AFFINE targets), gradient epilogue
     // (single-target rmse, weight_l2)
     int extra_launches() const { return (affine_ ? 2 : 0) + (post_ ? 1 : 0); }
+    // launches of one step() without the extra ones: gather, layer 1 and the head (one hidden layer: k_wide_one alone),
+    // five per further hidden layer, gradfin, update, advance
+    int base_launches() const { return m_.NH == 1 ? 4 : 3 + 5 * (m_.NH - 1) + 3; }
     // bytes of the exchange block a rank exposes in data-parallel mode: [2][xlen] floats + flags
     size_t dp_block_bytes() const { return (size_t)2 * dp_xlen() * sizeof(float) + 256; }
     int dp_xlen() const { return (m_.nflat + 16 + 31) / 32 * 32; }
@@ -92,11 +98,20 @@ private:
     cudaError_t ensure(int B);
     cudaError_t forward(const float* rec, const int* idx, long long rec_base, long long nrec, int B, int Bvalid,
                         const float* bscal, const float* pblock, cudaStream_t st);
+    // one hidden layer: k_wide_one over rows rec[idx[b]] (or rec[rec_base + b]), b < B, in mode ONE_TRAIN / ONE_STATS / ONE_EVAL
+    cudaError_t launch_one(int mode, const float* rec, const int* idx, long long rec_base, long long nrec, int B, const float* bscal,
+                           const float* pblock, float* yhat, float* parout, long long ldy, long long row0, double* evalstat,
+                           const float* shift_y, cudaStream_t st, int* grid_out);
+    int one_grid(int B) const;
+    cudaError_t finish_step(int n_head, int n_slab, const float* bscal, float* pblock, float* m, float* v, void* ost,
+                            float* grad, float* grad_final, float* loss_out, int apply, cudaStream_t st, const WideDp* dp);
     WideModel m_{};
     int cap_ = 0, mapB_ = 0, n_head_ = 0, n_slab_ = 0, ksplit_ = 1;
     bool persist_ = true;
     bool affine_ = false;      // some target is LOSS_AFFINE: statistics pass of the head kernel + k_stat_seeds per step
     bool post_ = false;        // single-target rmse or weight_l2: k_wide_gradpost finishes the flat gradient
+    void* one_fn_ = nullptr;   // one hidden layer: the k_wide_one instantiation of this model
+    int one_max_ = 0;          // its CTAs at most (resident CTAs per SM x SMs): rows of head_partial_ / colsum_[0] / evalpart_
     float* xb_ = nullptr;
     __nv_bfloat16* A_[8] = {nullptr};
     __nv_bfloat16* D_[2] = {nullptr, nullptr};

@@ -16,6 +16,8 @@
 // launches between the forward GEMMs and the training head: k_wide_head in its statistics mode over A_NH (sufficient
 // statistics of the batch's predictions per CTA) and k_stat_seeds (eh_stat_seeds.cuh: seed coefficients and loss value
 // into the batch's scalar row).
+// A chain with ONE hidden layer (33..512 units) replaces gather, layer 1, the GEMMs and the head by one exact-fp32 kernel,
+// k_wide_one (eh_wide_one.cuh), followed by the same k_wide_gradfin / k_wide_gradpost / k_wide_update.
 // Replaces Lux.Training.single_train_step! (src/training/epoch.jl:20-26) for wide chains; formulas: SURVEY 10.2-10.5.
 #pragma once
 #include <cuda_bf16.h>

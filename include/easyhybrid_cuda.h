@@ -80,7 +80,8 @@ typedef enum { EH_ROLE_NEURAL = 0, EH_ROLE_GLOBAL = 1, EH_ROLE_FIXED = 2 } eh_ro
 /* training losses of src/losses/loss_fn.jl:58-179.  The last three (and rmse over more than one target) depend on
  * statistics of the batch's PREDICTIONS (mean, variance, covariance with the observations): on the exact-fp32 kernels
  * their steps run a forward pre-pass over the batch first and take the one-launch-pair-per-step path (no persistent
- * kernel), on the tensor-core path (chains wider than 32) a statistics pass of the head kernel; single GPU on both.   */
+ * kernel), on the wide path (chains wider than 32) a statistics pass of the head kernel (one hidden layer: of
+ * k_wide_one); single GPU on both.   */
 typedef enum {
     EH_LOSS_MSE = 0, EH_LOSS_RMSE = 1, EH_LOSS_MAE = 2, EH_LOSS_NSELOSS = 3,
     EH_LOSS_PEARSONLOSS = 4, /* 1 - cor(yhat, y)                                                loss_fn.jl:75-77   */
@@ -331,7 +332,8 @@ eh_status eh_set_profiling(eh_ctx* ctx, int32_t on);
 
 /* which compiled kernel family serves this ctx (static string, never NULL), e.g.
  * "ffma2/PmRbQ10/P2/NH2/H16/O1/ACT_TANH/scale=true" (exact-fp32 register-tile kernels, specialised form),
- * "ffma2/PmProgram/..." (same kernels, process model interpreted per sample) or "wide/bf16-tcgen05".
+ * "ffma2/PmProgram/..." (same kernels, process model interpreted per sample), "wide/bf16-tcgen05" or, for one hidden layer
+ * of 33..512 units, "wide/fp32-one-hidden".
  * The reference has no counterpart; callers use it to report / assert the path a model took.          */
 const char* eh_kernel_variant(const eh_ctx* ctx);
 /* Plans `desc` as eh_create would and compiles its traced process model with NVRTC (EH_FLAG_JIT implied) WITHOUT touching a
