@@ -36,9 +36,11 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
         return fail(c, EH_EUNSUPPORTED,
                     "no fused kernel for this model: the register-tile kernels serve 1..3 hidden layers of summed width <= 32 "
                     "(all activations, <= 8 inputs, <= 2 outputs); the wide path serves 1..4 chains of equal depth, activation "
-                    "and input_batchnorm with <= 8 inputs and <= 2 outputs in total: one hidden layer of summed width 33..512 "
-                    "(exact fp32, all activations) or 2..6 hidden layers of summed width <= 512 per layer (bf16 tensor cores, "
-                    "tanh / sigmoid / relu) (got process_model=%d chains=%d inputs=%d hidden=%d x (<= %d) outputs=%d activation=%d)",
+                    "and input_batchnorm with <= 12 inputs and <= 4 outputs in total (more than 8 / 2 only with some layer "
+                    "wider than 32; 3..4 outputs: traced process models): one hidden layer of summed width 33..512 (exact fp32, "
+                    "all activations) or 2..6 hidden layers of summed width <= 512 per layer (bf16 tensor cores, tanh / "
+                    "sigmoid / relu) "
+                    "(got process_model=%d chains=%d inputs=%d hidden=%d x (<= %d) outputs=%d activation=%d)",
                     d->process_model, NC, P, NH, hmax, NOUT, c0.activation);
     // (one hidden layer: the fused exact-fp32 kernel k_wide_one, images padded to a multiple of 64 units)
     const int HP = NH == 1 ? eh::wide::WideNet::one_width(hmax) : eh::wide::WideNet::padded_width(hmax);

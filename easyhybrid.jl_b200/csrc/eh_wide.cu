@@ -62,6 +62,10 @@ cudaError_t gemm_prepare()
     if ((e = cudaFuncSetAttribute(k_wide_gemm_p<GEMM_BWD, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(k_wide_gemm_p<GEMM_FWD, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
     if ((e = cudaFuncSetAttribute(k_wide_gemm_p<GEMM_BWD, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
+    // (the layer-1 backward-data call of models with more than WIDE_MAXP inputs)
+    if ((e = cudaFuncSetAttribute(k_wide_gemm<GEMM_BWD, WIDE_MAXP_X>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem(GEMM_BWD))) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(k_wide_gemm_p<GEMM_BWD, 1, WIDE_MAXP_X>, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(k_wide_gemm_p<GEMM_BWD, 2, WIDE_MAXP_X>, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
     done = true;
     return cudaSuccess;
 }
@@ -83,7 +87,9 @@ cudaError_t gemm_bwd(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int
     GemmArgs g{};
     g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.aux = aux; g.out16 = out;
     g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn;
-    k_wide_gemm<GEMM_BWD><<<dim3(M / BM, N / gemm_bn(GEMM_BWD), 1), GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
+    const dim3 grid(M / BM, N / gemm_bn(GEMM_BWD), 1);
+    if (P1 > WIDE_MAXP) k_wide_gemm<GEMM_BWD, WIDE_MAXP_X><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
+    else k_wide_gemm<GEMM_BWD><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
     return cudaGetLastError();
 }
 // persistent forms (one CTA per SM, 128 x 256 tiles, double-buffered accumulator); tmW / tmWt must be built with
@@ -92,7 +98,7 @@ cudaError_t gemm_bwd(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int
 // single CTAs: the kernels are bound by shared-memory bandwidth -- TMA writes plus MMA operand reads -- not by L2 reads).
 static bool pg_cluster() { static const bool on = getenv("EH_WIDE_CLUSTER") != nullptr; return on; }
 int pg_box_rows() { return pg_cluster() ? PG_BN / 2 : PG_BN; }
-template <int MODE>
+template <int MODE, int PX = WIDE_MAXP>
 static cudaError_t launch_gemm_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& g, cudaStream_t st)
 {
     static int nsm = 0, max_clusters = -1;
@@ -116,20 +122,20 @@ static cudaError_t launch_gemm_p(const CUtensorMap& tmA, const CUtensorMap& tmB,
         if (max_clusters < 0) {
             cfg.gridDim = dim3((unsigned)(nsm & ~1));
             int mc = 0;
-            if (cudaOccupancyMaxActiveClusters(&mc, k_wide_gemm_p<MODE, 2>, &cfg) != cudaSuccess || mc < 1) { cudaGetLastError(); mc = 0; }
+            if (cudaOccupancyMaxActiveClusters(&mc, k_wide_gemm_p<MODE, 2, PX>, &cfg) != cudaSuccess || mc < 1) { cudaGetLastError(); mc = 0; }
             max_clusters = mc;
         }
         if (max_clusters > 0) {
             const int units = (mt / 2) * nn;
             const int ncl = std::min(std::min(max_clusters, nsm / 2), units);
             cfg.gridDim = dim3((unsigned)(2 * ncl));
-            return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 2>, tmA, tmB, g);
+            return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 2, PX>, tmA, tmB, g);
         }
         cfg.attrs = nullptr;
         cfg.numAttrs = 0;
     }
     cfg.gridDim = dim3((unsigned)std::min(mt * nn, nsm));
-    return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 1>, tmA, tmB, g);
+    return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 1, PX>, tmA, tmB, g);
 }
 int persistent_grid(int M, int N)
 {
@@ -156,6 +162,7 @@ cudaError_t gemm_bwd_p(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, i
     GemmArgs g{};
     g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.aux = aux; g.out16 = out;
     g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn;
+    if (P1 > WIDE_MAXP) return launch_gemm_p<GEMM_BWD, WIDE_MAXP_X>(tmD, tmWt, g, st);
     return launch_gemm_p<GEMM_BWD>(tmD, tmWt, g, st);
 }
 
@@ -181,8 +188,11 @@ struct HeadEntry { int pm, nout, scale, hch, aff; HeadKernel fn; };
 #define EH_HEAD_PMA(PMF, AFF) EH_HEAD(PMF, 1, 0, 1, AFF) EH_HEAD(PMF, 1, 1, 1, AFF) EH_HEAD(PMF, 2, 0, 1, AFF) EH_HEAD(PMF, 2, 1, 1, AFF) \
                               EH_HEAD(PMF, 1, 0, 2, AFF) EH_HEAD(PMF, 1, 1, 2, AFF) EH_HEAD(PMF, 2, 0, 2, AFF) EH_HEAD(PMF, 2, 1, 2, AFF)
 #define EH_HEAD_PM(PMF) EH_HEAD_PMA(PMF, 0) EH_HEAD_PMA(PMF, 1)
+// three and four outputs: traced process models only (the built-in forms have two parameters)
+#define EH_HEAD_PMA34(PMF, AFF) EH_HEAD(PMF, 3, 0, 1, AFF) EH_HEAD(PMF, 3, 1, 1, AFF) EH_HEAD(PMF, 4, 0, 1, AFF) EH_HEAD(PMF, 4, 1, 1, AFF) \
+                                EH_HEAD(PMF, 3, 0, 2, AFF) EH_HEAD(PMF, 3, 1, 2, AFF) EH_HEAD(PMF, 4, 0, 2, AFF) EH_HEAD(PMF, 4, 1, 2, AFF)
 const HeadEntry g_heads[] = {EH_HEAD_PM(PmRbQ10) EH_HEAD_PM(PmExpo) EH_HEAD_PM(PmLinear) EH_HEAD_PM(PmLinear2) EH_HEAD_PM(PmExpo2)
-                             EH_HEAD_PM(PmProgram)};
+                             EH_HEAD_PM(PmProgram) EH_HEAD_PMA34(PmProgram, 0) EH_HEAD_PMA34(PmProgram, 1)};
 
 // aff: the training head of a model with LOSS_AFFINE targets (the statistics and evaluation modes take aff = 0)
 HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false)
@@ -192,18 +202,20 @@ HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false)
     return nullptr;
 }
 
-// the fused kernel of one hidden layer: one instantiation per process model, output count and scale_nn_outputs
-// (activation, input count, mode and loss kinds are run-time arguments)
+// the fused kernel of one hidden layer: one instantiation per process model, output count, scale_nn_outputs and input
+// bound (one_px: 8, or 12 for models with 9..12 inputs); activation, input count, mode and loss kinds are run-time arguments
 typedef void (*OneKernel)(const OneArgs);
-struct OneEntry { int pm, nout, scale; OneKernel fn; };
-#define EH_ONE(PMF, NOUT, SCALE) {PMF::ID, NOUT, SCALE, k_wide_one<HeadCfg<PMF, NOUT, (SCALE != 0)>>},
-#define EH_ONE_PM(PMF) EH_ONE(PMF, 1, 0) EH_ONE(PMF, 1, 1) EH_ONE(PMF, 2, 0) EH_ONE(PMF, 2, 1)
-const OneEntry g_ones[] = {EH_ONE_PM(PmRbQ10) EH_ONE_PM(PmExpo) EH_ONE_PM(PmLinear) EH_ONE_PM(PmLinear2) EH_ONE_PM(PmExpo2)
-                           EH_ONE_PM(PmProgram)};
-OneKernel find_one(int pm, int nout, int scale)
+struct OneEntry { int pm, nout, scale, px; OneKernel fn; };
+#define EH_ONE(PMF, NOUT, SCALE, PX) {PMF::ID, NOUT, SCALE, PX, k_wide_one<HeadCfg<PMF, NOUT, (SCALE != 0)>, PX>},
+#define EH_ONE_PM(PMF, PX) EH_ONE(PMF, 1, 0, PX) EH_ONE(PMF, 1, 1, PX) EH_ONE(PMF, 2, 0, PX) EH_ONE(PMF, 2, 1, PX)
+#define EH_ONE_PM34(PMF, PX) EH_ONE(PMF, 3, 0, PX) EH_ONE(PMF, 3, 1, PX) EH_ONE(PMF, 4, 0, PX) EH_ONE(PMF, 4, 1, PX)
+#define EH_ONE_ALL(PX) EH_ONE_PM(PmRbQ10, PX) EH_ONE_PM(PmExpo, PX) EH_ONE_PM(PmLinear, PX) EH_ONE_PM(PmLinear2, PX) \
+                       EH_ONE_PM(PmExpo2, PX) EH_ONE_PM(PmProgram, PX) EH_ONE_PM34(PmProgram, PX)
+const OneEntry g_ones[] = {EH_ONE_ALL(WIDE_MAXP) EH_ONE_ALL(WIDE_MAXP_X)};
+OneKernel find_one(int pm, int nout, int scale, int P)
 {
     for (const OneEntry& e : g_ones)
-        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0)) return e.fn;
+        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0) && e.px == one_px(P)) return e.fn;
     return nullptr;
 }
 
@@ -229,12 +241,15 @@ WideDims dims_of(const WideModel& m)
 
 bool WideNet::supported(int P, int hmax, int NH, int NOUT, int act, int pm)
 {
+    // 9..12 inputs and 3..4 outputs only where some layer is wider than 32 units: a narrower model (the exact path's, or
+    // here under EH_NO_SMALL_PROGRAM) keeps the limits it always had
+    const int pmax = hmax > 32 ? WIDE_MAXP_X : WIDE_MAXP, omax = hmax > 32 ? 4 : 2;
     if (NH == 1) {   // (one layer of <= 32 units belongs to the register-tile kernels)
-        if (P < 1 || P > WIDE_MAXP || NOUT < 1 || NOUT > 2 || hmax <= 32 || hmax > 512) return false;
+        if (P < 1 || P > pmax || NOUT < 1 || NOUT > omax || hmax <= 32 || hmax > 512) return false;
         if (act != ACT_TANH && act != ACT_SIGMOID && act != ACT_RELU && act != ACT_IDENTITY && act != ACT_SWISH) return false;
-        return find_one(pm, NOUT, 0) != nullptr;
+        return find_one(pm, NOUT, 0, P) != nullptr;
     }
-    if (P < 1 || P > WIDE_MAXP || NH < 2 || NH > 6 || NOUT < 1 || NOUT > 2) return false;
+    if (P < 1 || P > pmax || NH < 2 || NH > 6 || NOUT < 1 || NOUT > omax) return false;
     if (hmax < 1 || hmax > 512) return false;
     if (act != ACT_TANH && act != ACT_SIGMOID && act != ACT_RELU && act != ACT_IDENTITY) return false;
     return find_head(pm, NOUT, 0, padded_width(hmax) / 256) != nullptr;
@@ -255,8 +270,8 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
     if (m.NH == 1) {
         // one hidden layer: no GEMM images, tensor maps, activation buffers or head kernel; k_wide_one's partial buffers
         // have one row per CTA it can keep resident
-        OneKernel ok = find_one(m.pm, m.NOUT, m.scale);
-        if (!ok || m.H % 64 || m.H > 512 || m.R4 > WIDE_MAXP + ONE_FY) {
+        OneKernel ok = find_one(m.pm, m.NOUT, m.scale, m.P);
+        if (!ok || m.H % 64 || m.H > 512 || m.P > WIDE_MAXP_X || m.R4 > one_px(m.P) + ONE_FY) {
             snprintf(err, errlen, "wide path: no fused one-hidden-layer kernel for this process model / shape");
             delete w;
             return nullptr;
@@ -298,10 +313,10 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
         const size_t cs = (size_t)w->one_max_ * (1 + m.P) * m.H * 4;
         if ((e = cudaMalloc(&w->colsum_[0], cs)) != cudaSuccess) return bail("cudaMalloc", e);
     }
-    if ((e = cudaMalloc(&w->W1img_, (size_t)WIDE_MAXP * m.H * 4)) != cudaSuccess) return bail("cudaMalloc", e);
+    if ((e = cudaMalloc(&w->W1img_, (size_t)WIDE_MAXP_X * m.H * 4)) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&w->WOimg_, (size_t)4 * m.H * 4)) != cudaSuccess) return bail("cudaMalloc", e);
     if ((e = cudaMalloc(&w->BOimg_, 16)) != cudaSuccess) return bail("cudaMalloc", e);
-    cudaMemset(w->W1img_, 0, (size_t)WIDE_MAXP * m.H * 4);
+    cudaMemset(w->W1img_, 0, (size_t)WIDE_MAXP_X * m.H * 4);
     cudaMemset(w->WOimg_, 0, (size_t)4 * m.H * 4);
     cudaMemset(w->BOimg_, 0, 16);
     {
@@ -326,7 +341,7 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
         if ((e = cudaMalloc(&w->d_prog_, sizeof pd)) != cudaSuccess) return bail("cudaMalloc", e);
         if ((e = cudaMemcpy(w->d_prog_, &pd, sizeof pd, cudaMemcpyHostToDevice)) != cudaSuccess) return bail("cudaMemcpy", e);
     }
-    w->n_head_ = m.NH == 1 ? w->one_max_ : 3 * m.nsm;   // three CTAs of the head kernel are resident per SM (80 registers)
+    w->n_head_ = m.NH == 1 ? w->one_max_ : head_ctas_per_sm(m.NOUT) * m.nsm;   // resident CTAs of the head kernel (k_wide_head)
     if (cudaStreamCreateWithFlags(&w->side_, cudaStreamNonBlocking) != cudaSuccess || cudaEventCreateWithFlags(&w->ev_wgrad_, cudaEventDisableTiming) != cudaSuccess ||
         cudaEventCreateWithFlags(&w->ev_wred_, cudaEventDisableTiming) != cudaSuccess) {
         cudaGetLastError();
@@ -432,7 +447,8 @@ cudaError_t WideNet::forward(const float* rec, const int* idx, long long rec_bas
         const unsigned g1 = (unsigned)((B + rows_per_cta - 1) / rows_per_cta);
         if (d.P <= 2) k_wide_first<2><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
         else if (d.P <= 4) k_wide_first<4><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
-        else k_wide_first<8><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
+        else if (d.P <= WIDE_MAXP) k_wide_first<8><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
+        else k_wide_first<WIDE_MAXP_X><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
     }
     WN(cudaGetLastError());
     for (int l = 2; l <= m_.NH; l++) {

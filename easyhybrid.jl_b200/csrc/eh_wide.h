@@ -58,7 +58,8 @@ struct WideModel {          // filled by eh_lib's planner from the model descrip
 // the wide-chain training step: owns activations / deltas / bf16 weight images / partial buffers
 class WideNet {
 public:
-    // hmax: widest embedded hidden layer (padded up to 256 or 512 inside; one hidden layer: to a multiple of 64)
+    // hmax: widest embedded hidden layer (padded up to 256 or 512 inside; one hidden layer: to a multiple of 64).
+    // P <= 12 inputs and NOUT <= 4 outputs (3..4: traced process models) when hmax > 32, else P <= 8 and NOUT <= 2
     static bool supported(int P, int hmax, int NH, int NOUT, int act, int pm);
     static int padded_width(int hmax) { return hmax <= 256 ? 256 : 512; }
     // one hidden layer of 33..512 units (any activation, swish included) trains in the fused exact-fp32 kernel k_wide_one

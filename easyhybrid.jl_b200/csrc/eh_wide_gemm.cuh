@@ -27,7 +27,8 @@ namespace eh {
 namespace wide {
 
 constexpr int BM = 128, BK = 64, UMMA_K = 16;
-constexpr int WIDE_MAXP = 8;          // chain inputs (all chains together) the tensor-core path takes
+constexpr int WIDE_MAXP = 8;          // chain inputs (all chains together) the kernels of every wide model are built for
+constexpr int WIDE_MAXP_X = 12;       // ... and the separate instantiations of models with 9..12 inputs (summed width > 32)
 constexpr int BS_BN_OFF = 3 * MAXT;   // == BS_BN of eh_chunk.cuh (per-batch scalar row: input BatchNorm mu / rstd)
 constexpr int GEMM_THREADS = 192;            // warp 0: TMA, warp 1: MMA + TMEM alloc, warps 2..5: epilogue
 // Tile width and pipeline depth per GEMM kind.
@@ -184,7 +185,9 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
 
 // grid: (M / BM, N / BN, ksplits).  FWD / BWD: tmA = [M x K] K-major (box 64 x 128), tmB = [N x K] K-major
 // (box 64 x 128).  WGRAD: tmA = deltas [Kall x M], tmB = activations [Kall x N], both MN-major (box 64 x 64).
-template <int MODE>
+// PX: chain inputs the backward-data epilogue's input-weighted column sums hold (WIDE_MAXP, or WIDE_MAXP_X in the
+// instantiation that serves the layer-1 call of models with more than WIDE_MAXP inputs)
+template <int MODE, int PX = WIDE_MAXP>
 __global__ void __launch_bounds__(GEMM_THREADS, MODE == GEMM_WGRAD ? 1 : 2)
 k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g)
 {
@@ -340,10 +343,10 @@ k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
         if (MODE == GEMM_BWD && g.colsum != nullptr) {
             // column sums over this warp's 32 rows, straight from the staged bf16 strip: lane l owns columns 4l .. 4l+3
             __syncwarp();
-            float cs[4] = {0.f, 0.f, 0.f, 0.f}, cw[WIDE_MAXP][4];
-            float xr[WIDE_MAXP] = {0.f};
+            float cs[4] = {0.f, 0.f, 0.f, 0.f}, cw[PX][4];
+            float xr[PX] = {0.f};
 #pragma unroll
-            for (int p = 0; p < WIDE_MAXP; p++) {
+            for (int p = 0; p < PX; p++) {
                 cw[p][0] = cw[p][1] = cw[p][2] = cw[p][3] = 0.f;
                 if (p < g.P1) {
                     float x = g.xb[(size_t)row * g.R4 + p];
@@ -358,7 +361,7 @@ k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 const float2 f1 = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&v.y));
                 cs[0] += f0.x; cs[1] += f0.y; cs[2] += f1.x; cs[3] += f1.y;
 #pragma unroll
-                for (int p = 0; p < WIDE_MAXP; p++) {
+                for (int p = 0; p < PX; p++) {
                     if (p < g.P1) {
                         const float x = __shfl_sync(0xffffffffu, xr[p], r);
                         cw[p][0] = fmaf(f0.x, x, cw[p][0]); cw[p][1] = fmaf(f0.y, x, cw[p][1]);
@@ -367,15 +370,16 @@ k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                 }
             }
             // combine the four warps (fixed order) so that one 128-row slab per CTA goes out
-            float* s_cs = reinterpret_cast<float*>(gen_base + 4 * (32 * OPITCH));   // [4 warps][1 + WIDE_MAXP][BN], behind the strips
-            *reinterpret_cast<float4*>(s_cs + (q * (1 + WIDE_MAXP) + 0) * BN + lane * 4) = make_float4(cs[0], cs[1], cs[2], cs[3]);
+            float* s_cs = reinterpret_cast<float*>(gen_base + 4 * (32 * OPITCH));   // [4 warps][1 + PX][BN], behind the strips
+            static_assert(4 * 32 * OPITCH + 4 * (1 + PX) * BN * 4 <= STAGES * STAGE_BYTES, "column sums fit the idle stages");
+            *reinterpret_cast<float4*>(s_cs + (q * (1 + PX) + 0) * BN + lane * 4) = make_float4(cs[0], cs[1], cs[2], cs[3]);
 #pragma unroll
-            for (int p = 0; p < WIDE_MAXP; p++)
-                if (p < g.P1) *reinterpret_cast<float4*>(s_cs + (q * (1 + WIDE_MAXP) + 1 + p) * BN + lane * 4) = make_float4(cw[p][0], cw[p][1], cw[p][2], cw[p][3]);
+            for (int p = 0; p < PX; p++)
+                if (p < g.P1) *reinterpret_cast<float4*>(s_cs + (q * (1 + PX) + 1 + p) * BN + lane * 4) = make_float4(cw[p][0], cw[p][1], cw[p][2], cw[p][3]);
             asm volatile("bar.sync 1, 128;" ::: "memory");
             const int t = (warp - 2) * 32 + lane;   // column of the tile
             for (int p = 0; p <= g.P1; p++) {
-                const float v = ((s_cs[(0 * (1 + WIDE_MAXP) + p) * BN + t] + s_cs[(1 * (1 + WIDE_MAXP) + p) * BN + t]) + s_cs[(2 * (1 + WIDE_MAXP) + p) * BN + t]) + s_cs[(3 * (1 + WIDE_MAXP) + p) * BN + t];
+                const float v = ((s_cs[(0 * (1 + PX) + p) * BN + t] + s_cs[(1 * (1 + PX) + p) * BN + t]) + s_cs[(2 * (1 + PX) + p) * BN + t]) + s_cs[(3 * (1 + PX) + p) * BN + t];
                 g.colsum[((size_t)blockIdx.x * (1 + g.P1) + p) * g.N + n0 + t] = v;
             }
         }
@@ -454,12 +458,14 @@ __device__ __forceinline__ void cluster_sync_all()
 // weight tile of a stage (128 of the 256 rows) and multicasts it into both, so a tile costs 256 KB of L2 reads instead of
 // 384 KB -- the kernel runs at the L2 throughput limit (about 12 TB/s), not at the tensor pipe's.  A stage is reusable
 // when BOTH CTAs' MMAs have read it (the commits arrive on both empty barriers).  tmB: box of BN rows for CL = 1, BN / 2 for CL = 2.
-template <int MODE, int CL>
+// PX: as for k_wide_gemm (the staged strip of a warp, 32 x PG_OPITCH bytes, holds the (1 + PX) x PG_CW parked sums)
+template <int MODE, int CL, int PX = WIDE_MAXP>
 __global__ void __launch_bounds__(PG_THREADS, 1)
 k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g)
 {
     static_assert(MODE == GEMM_FWD || MODE == GEMM_BWD, "persistent form serves forward and backward-data");
     static_assert(CL == 1 || CL == 2, "cluster of one or two CTAs");
+    static_assert((1 + PX) * PG_CW * 4 <= 32 * PG_OPITCH, "parked column sums fit the staged strip");
     constexpr int BN = PG_BN, STAGES = PG_STAGES, STAGE_BYTES = PG_STAGE_BYTES, A_STAGE_BYTES = BM * BK * 2;
     constexpr int STG_OFF = STAGES * STAGE_BYTES, SIDE_OFF = STG_OFF + PG_STG_BYTES, BAR_OFF = SIDE_OFF + PG_SIDE_BYTES;
     extern __shared__ uint8_t smem_raw[];
@@ -635,13 +641,13 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
             // BWD: column sums over this warp's 32 rows, straight from the staged strip (lane l owns columns NCC l .. NCC l + NCC - 1)
             // (the input-weighted sums exist for the layer-1 call only; the loop is specialised on their count -- unrolled over
             // WIDE_MAXP with a run-time bound it cost 1 000 mostly predicated-off instructions per tile and warp)
-            float cs[NCC], cw[WIDE_MAXP][NCC];
+            float cs[NCC], cw[PX][NCC];
             const bool want_cs = MODE == GEMM_BWD && g.colsum != nullptr;
             if (want_cs) {
 #pragma unroll
                 for (int k = 0; k < NCC; k++) cs[k] = 0.f;
 #pragma unroll
-                for (int p = 0; p < WIDE_MAXP; p++)
+                for (int p = 0; p < PX; p++)
 #pragma unroll
                     for (int k = 0; k < NCC; k++) cw[p][k] = 0.f;
                 auto colsums = [&](auto pn_c) {
@@ -675,11 +681,15 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
                         }
                     }
                 };
-                if (g.P1 == 0) colsums(std::integral_constant<int, 0>{});
-                else if (g.P1 == 1) colsums(std::integral_constant<int, 1>{});
-                else if (g.P1 == 2) colsums(std::integral_constant<int, 2>{});
-                else if (g.P1 <= 4) colsums(std::integral_constant<int, 4>{});
-                else colsums(std::integral_constant<int, WIDE_MAXP>{});
+                if constexpr (PX > WIDE_MAXP) {
+                    colsums(std::integral_constant<int, PX>{});   // (launched for layer 1 of a model with > WIDE_MAXP inputs)
+                } else {
+                    if (g.P1 == 0) colsums(std::integral_constant<int, 0>{});
+                    else if (g.P1 == 1) colsums(std::integral_constant<int, 1>{});
+                    else if (g.P1 == 2) colsums(std::integral_constant<int, 2>{});
+                    else if (g.P1 <= 4) colsums(std::integral_constant<int, 4>{});
+                    else colsums(std::integral_constant<int, WIDE_MAXP>{});
+                }
             }
             __syncwarp();
             // CW bf16 per row = LPR lanes of 16 bytes: RPI rows per instruction
@@ -697,7 +707,7 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
                 for (int k = 0; k < NCC; k++) mine[lane * NCC + k] = cs[k];
 #pragma unroll
-                for (int p = 0; p < WIDE_MAXP; p++)
+                for (int p = 0; p < PX; p++)
                     if (p < g.P1) {
 #pragma unroll
                         for (int k = 0; k < NCC; k++) mine[(1 + p) * CW + lane * NCC + k] = cw[p][k];

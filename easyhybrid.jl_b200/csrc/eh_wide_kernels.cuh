@@ -1,6 +1,6 @@
 // eh_wide_kernels.cuh -- the non-GEMM kernels of the wide-hidden-layer training step (sm_100a).
 //
-// One optimiser step of a hybrid model whose Dense chain is  P -> H -> ... -> H -> NOUT  with H >= 256
+// One optimiser step of a hybrid model whose Dense chain is  P -> H -> ... -> H -> NOUT  with H >= 256 (P <= 12, NOUT <= 4)
 // (BASELINE config 5: 3 x 512) is a sequence of launches on one stream:
 //   k_wide_gather    batch records (AoS, gathered through the index stream) -> compact batch
 //   k_wide_first     layer 1 (fan-in P is tiny: elementwise)          A_1 = act(W_1 x + b_1)        bf16
@@ -77,7 +77,7 @@ __device__ __forceinline__ uint32_t pack2(float lo, float hi) { return pack_bf16
 // A thread owns 8 consecutive outputs (their weights stay in registers) and walks FIRST_ROWS rows of the batch;
 // a CTA covers the whole width for 256 / (H / 8) row groups.
 constexpr int FIRST_ROWS = 16;
-// PMAX: compile-time bound on the chain inputs (2 / 4 / 8) -- the weights a thread keeps in registers.  Rows go four at
+// PMAX: compile-time bound on the chain inputs (2 / 4 / 8 / 12) -- the weights a thread keeps in registers.  Rows go four at
 // a time with their inputs loaded first: the kernel is a stream of 16-byte stores (H bf16 per row) and must not wait for
 // one L2 round trip per row.
 template <int PMAX>
@@ -159,9 +159,12 @@ struct HeadArgs {
 };
 
 // ---- output layer + physics + loss seeds + backward into D_NH; one warp per sample row, 8 warps per CTA ----
-// H / 256 chunks of 8 consecutive features per lane (16-byte bf16 accesses).
+// H / 256 chunks of 8 consecutive features per lane (16-byte bf16 accesses).  Three CTAs per SM (80 registers); the
+// three- and four-output instantiations (traced process models) hold up to 64 gradient accumulators and run at two
+// (head_ctas_per_sm).
+__host__ __device__ constexpr int head_ctas_per_sm(int NOUT) { return NOUT > 2 ? 2 : 3; }
 template <class HC, int HCH>
-__global__ void __launch_bounds__(256, 3) k_wide_head(const HeadArgs a)
+__global__ void __launch_bounds__(256, head_ctas_per_sm(HC::NOUT)) k_wide_head(const HeadArgs a)
 {
     using PM = typename HC::PM;
     constexpr int NOUT = HC::NOUT, T = HC::T, F = HC::F, NPS = HC::NPS;

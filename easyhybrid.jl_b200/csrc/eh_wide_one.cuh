@@ -1,6 +1,6 @@
 // eh_wide_one.cuh -- one training step of a chain with ONE wide hidden layer (33..512 units), exact fp32, one kernel (sm_100a).
 //
-// With one hidden layer there is no H x H contraction: layer 1 has fan-in P <= 8 and the output layer fan-out NOUT <= 2,
+// With one hidden layer there is no H x H contraction: layer 1 has fan-in P <= 12 and the output layer fan-out NOUT <= 4,
 // so the whole forward, the loss seeds, the backward and the gradient sums are per-sample work on CUDA cores.  k_wide_one
 // does all of it on-chip and reads nothing per step but the batch records; it replaces k_wide_gather, k_wide_first, the
 // forward / backward GEMMs and k_wide_head of the NH >= 2 path.  What follows it is the wide path's unchanged tail:
@@ -41,12 +41,15 @@ enum : int { ONE_TRAIN = 0, ONE_STATS = 1, ONE_EVAL = 2 };
 __host__ __device__ constexpr int one_group_threads(int H) { return H / 2; }
 __host__ __device__ constexpr int one_block(int H) { return ONE_THREADS / (H / 2) * (H / 2); }
 __host__ __device__ constexpr int one_tile_rows(int H) { return ONE_THREADS / (H / 2) * ONE_R; }
-// dynamic shared memory: three record buffers [3][tile rows][WIDE_MAXP + ONE_FY], reused after the row loop for the CTA
+// chain inputs an instantiation holds: WIDE_MAXP, or WIDE_MAXP_X for models with 9..12 inputs (their own instantiations:
+// the weights and gradient accumulators of 12 inputs do not fit the register budget of the 8-input kernel)
+__host__ __device__ constexpr int one_px(int P) { return P > WIDE_MAXP ? WIDE_MAXP_X : WIDE_MAXP; }
+// dynamic shared memory: three record buffers [3][tile rows][PX + ONE_FY], reused after the row loop for the CTA
 // reduction of the unit accumulators [groups][NOUT + 1 + P][H]
 __host__ __device__ constexpr int one_smem(int H, int P, int NOUT)
 {
-    return 4 * (3 * one_tile_rows(H) * (WIDE_MAXP + ONE_FY) > (ONE_THREADS / (H / 2)) * (NOUT + 1 + P) * H
-                    ? 3 * one_tile_rows(H) * (WIDE_MAXP + ONE_FY)
+    return 4 * (3 * one_tile_rows(H) * (one_px(P) + ONE_FY) > (ONE_THREADS / (H / 2)) * (NOUT + 1 + P) * H
+                    ? 3 * one_tile_rows(H) * (one_px(P) + ONE_FY)
                     : (ONE_THREADS / (H / 2)) * (NOUT + 1 + P) * H);
 }
 
@@ -104,10 +107,10 @@ __device__ __forceinline__ float one_xsum8(float (&v)[8], int lane)
     return v[0];
 }
 
-// forward of a thread's two units over its group's ONE_R rows.  xs: the group's rows of the tile, [ONE_R][WIDE_MAXP]
-// normalised inputs (zero beyond P); s_pw: this warp's [2][ONE_R] output-layer sums
-template <int ACT, int PMAX, int NOUT>
-__device__ __forceinline__ void one_forward(const float* xs, const float2 (&w1)[WIDE_MAXP], float2 b1, const float2 (&wo)[2],
+// forward of a thread's two units over its group's ONE_R rows.  xs: the group's rows of the tile, [ONE_R][PX]
+// normalised inputs (zero beyond P); s_pw: this warp's [NO][ONE_R] output-layer sums (NO = max(NOUT, 2))
+template <int ACT, int PMAX, int NOUT, int PX, int NO>
+__device__ __forceinline__ void one_forward(const float* xs, const float2 (&w1)[PX], float2 b1, const float2 (&wo)[NO],
                                             float2 (&A)[ONE_R], float2 (&Gd)[ONE_R], float* s_pw, int lane)
 {
 #pragma unroll
@@ -119,7 +122,7 @@ __device__ __forceinline__ void one_forward(const float* xs, const float2 (&w1)[
             float x[PMAX];
 #pragma unroll
             for (int q = 0; q < PMAX; q += 2) {
-                const float2 v = *reinterpret_cast<const float2*>(xs + r * WIDE_MAXP + q);
+                const float2 v = *reinterpret_cast<const float2*>(xs + r * PX + q);
                 x[q] = v.x;
                 if (q + 1 < PMAX) x[q + 1] = v.y;
             }
@@ -141,19 +144,23 @@ __device__ __forceinline__ void one_forward(const float* xs, const float2 (&w1)[
     }
 }
 
-template <int ACT, int NOUT>
-__device__ __forceinline__ void one_forward_p(int P, const float* xs, const float2 (&w1)[WIDE_MAXP], float2 b1, const float2 (&wo)[2],
+template <int ACT, int NOUT, int PX, int NO>
+__device__ __forceinline__ void one_forward_p(int P, const float* xs, const float2 (&w1)[PX], float2 b1, const float2 (&wo)[NO],
                                               float2 (&A)[ONE_R], float2 (&Gd)[ONE_R], float* s_pw, int lane)
 {
-    if (P <= 2) one_forward<ACT, 2, NOUT>(xs, w1, b1, wo, A, Gd, s_pw, lane);
-    else if (P <= 4) one_forward<ACT, 4, NOUT>(xs, w1, b1, wo, A, Gd, s_pw, lane);
-    else one_forward<ACT, 8, NOUT>(xs, w1, b1, wo, A, Gd, s_pw, lane);
+    if constexpr (PX > WIDE_MAXP) {
+        one_forward<ACT, PX, NOUT, PX, NO>(xs, w1, b1, wo, A, Gd, s_pw, lane);   // (9..12 inputs)
+    } else {
+        if (P <= 2) one_forward<ACT, 2, NOUT, PX, NO>(xs, w1, b1, wo, A, Gd, s_pw, lane);
+        else if (P <= 4) one_forward<ACT, 4, NOUT, PX, NO>(xs, w1, b1, wo, A, Gd, s_pw, lane);
+        else one_forward<ACT, 8, NOUT, PX, NO>(xs, w1, b1, wo, A, Gd, s_pw, lane);
+    }
 }
 
 // backward of a thread's two units over its group's rows: delta = act'(z) sum_o Wo[o] dz_o -> dW1, db1, dWo
-template <int PMAX, int NOUT>
-__device__ __forceinline__ void one_backward(const float* xs, const float* s_dzg, const float2 (&wo)[2], const float2 (&A)[ONE_R],
-                                             const float2 (&Gd)[ONE_R], float2 (&gW1)[WIDE_MAXP], float2& gb, float2 (&gWo)[2])
+template <int PMAX, int NOUT, int PX, int NO>
+__device__ __forceinline__ void one_backward(const float* xs, const float* s_dzg, const float2 (&wo)[NO], const float2 (&A)[ONE_R],
+                                             const float2 (&Gd)[ONE_R], float2 (&gW1)[PX], float2& gb, float2 (&gWo)[NO])
 {
 #pragma unroll
     for (int r = 0; r < ONE_R; r++) {
@@ -167,7 +174,7 @@ __device__ __forceinline__ void one_backward(const float* xs, const float* s_dzg
         gb = add2(gb, dl);
 #pragma unroll
         for (int q = 0; q < PMAX; q += 2) {
-            const float2 v = *reinterpret_cast<const float2*>(xs + r * WIDE_MAXP + q);
+            const float2 v = *reinterpret_cast<const float2*>(xs + r * PX + q);
             gW1[q] = fma2s(dl, v.x, gW1[q]);
             if (q + 1 < PMAX) gW1[q + 1] = fma2s(dl, v.y, gW1[q + 1]);
         }
@@ -176,11 +183,15 @@ __device__ __forceinline__ void one_backward(const float* xs, const float* s_dzg
     }
 }
 
-template <class HC>
-__global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
+// PX: chain inputs held (one_px).  The instantiations of 9..12 inputs or 3..4 outputs (traced process models) keep more
+// weights and accumulators in registers than the 128 of two resident CTAs allow: they run at one CTA per SM.
+template <class HC, int PX = WIDE_MAXP>
+__global__ void __launch_bounds__(ONE_THREADS, (PX > WIDE_MAXP || HC::NOUT > 2) ? 1 : 2) k_wide_one(const OneArgs a)
 {
     using PM = typename HC::PM;
     constexpr int NOUT = HC::NOUT, T = HC::T, F = HC::F, NPS = HC::NPS;
+    constexpr int NO = NOUT > 2 ? NOUT : 2;            // output-layer registers / shared rows (two for one output, as before)
+    constexpr int NPRE = (PX + ONE_FY) / 2;            // record floats a thread fetches per tile, at most (16 R4 / (H / 2))
     constexpr int MAXRT = ONE_THREADS / 32 * ONE_R;   // tile rows at most (H = 64)
     const int H = a.d.H, P = a.d.P, R4 = a.d.R4;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
@@ -188,23 +199,23 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
     const int grp = tid / NTg, u0 = 2 * (tid - grp * NTg);   // my group, my two units
     __shared__ float s_pms[MAXPS * PMS_PER_SLOT + MAXPS];
     __shared__ PmProgData s_prog;
-    __shared__ float s_bn[2 * WIDE_MAXP];
-    __shared__ float s_part[ONE_THREADS / 32][2 * ONE_R];   // per warp: output-layer sums of its group's rows
-    __shared__ float s_dz[2 * MAXRT];                        // [NOUT][tile rows] output-layer deltas
+    __shared__ float s_bn[2 * PX];
+    __shared__ float s_part[ONE_THREADS / 32][NO * ONE_R];  // per warp: output-layer sums of its group's rows
+    __shared__ float s_dz[NO * MAXRT];                       // [NOUT][tile rows] output-layer deltas
     __shared__ double s_e[ONE_THREADS / 32][MAXT * 8];      // statistics / eval: sufficient statistics per warp
     __shared__ float s_red[ONE_THREADS / 32][16];
-    extern __shared__ float s_dyn[];                         // [3][tile rows][WIDE_MAXP + ONE_FY] records, then the reduction
-    float* s_x = s_dyn;                                      // [3][RT][WIDE_MAXP] normalised chain inputs (zero beyond P)
-    float* s_fy = s_dyn + 3 * RT * WIDE_MAXP;                // [3][RT][ONE_FY] forcings then targets
+    extern __shared__ float s_dyn[];                         // [3][tile rows][PX + ONE_FY] records, then the reduction
+    float* s_x = s_dyn;                                      // [3][RT][PX] normalised chain inputs (zero beyond P)
+    float* s_fy = s_dyn + 3 * RT * PX;                       // [3][RT][ONE_FY] forcings then targets
     for (int i = tid; i < MAXPS * PMS_PER_SLOT + MAXPS; i += blockDim.x) s_pms[i] = a.pblock[a.d.nflat + i];
     if (PM::DYNAMIC) {
         const int* src = reinterpret_cast<const int*>(a.prog);
         int* dst = reinterpret_cast<int*>(&s_prog);
         for (int i = tid; i < (int)(sizeof(PmProgData) / 4); i += blockDim.x) dst[i] = src[i];
     }
-    if (tid < 2 * WIDE_MAXP) s_bn[tid] = (a.use_bn && tid < 2 * P) ? a.bscal[BS_BN + tid] : ((tid & 1) ? 1.f : 0.f);
+    if (tid < 2 * PX) s_bn[tid] = (a.use_bn && tid < 2 * P) ? a.bscal[BS_BN + tid] : ((tid & 1) ? 1.f : 0.f);
     for (int i = tid; i < ONE_THREADS / 32 * MAXT * 8; i += blockDim.x) (&s_e[0][0])[i] = 0.0;
-    for (int i = tid; i < 3 * RT * WIDE_MAXP; i += blockDim.x) s_x[i] = 0.f;
+    for (int i = tid; i < 3 * RT * PX; i += blockDim.x) s_x[i] = 0.f;
     const int nf = PM::DYNAMIC ? a.nf : F, nt = PM::DYNAMIC ? a.nt : T;
     PmCtx cx;
     cx.pms = s_pms + MAXPS;
@@ -219,16 +230,16 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
         if (s >= NPS || a.slot[s].role != ROLE_NEURAL) cx.uniform_mask |= 1u << s;
 
     // my units' weights (registers) and the accumulators of their gradient
-    float2 w1[WIDE_MAXP], wo[2], gW1[WIDE_MAXP], gWo[2];
+    float2 w1[PX], wo[NO], gW1[PX], gWo[NO];
     const float2 b1 = f2(__ldg(a.b1img + u0), __ldg(a.b1img + u0 + 1));
     float2 gb = f2s(0.f);
 #pragma unroll
-    for (int p = 0; p < WIDE_MAXP; p++) {
+    for (int p = 0; p < PX; p++) {
         w1[p] = p < P ? f2(__ldg(a.W1img + (size_t)p * H + u0), __ldg(a.W1img + (size_t)p * H + u0 + 1)) : f2s(0.f);
         gW1[p] = f2s(0.f);
     }
 #pragma unroll
-    for (int o = 0; o < 2; o++) {
+    for (int o = 0; o < NO; o++) {
         wo[o] = o < NOUT ? f2(__ldg(a.WOimg + (size_t)o * H + u0), __ldg(a.WOimg + (size_t)o * H + u0 + 1)) : f2s(0.f);
         gWo[o] = f2s(0.f);
     }
@@ -240,12 +251,12 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
 #pragma unroll
     for (int q = 0; q < MAXPS; q++) gphi[q] = 0.f;
 
-    // records of a tile: up to 8 floats per thread in flight (16 R4 / (H / 2) <= 8), stored after the forward of the tile before
+    // records of a tile: up to NPRE floats per thread in flight (16 R4 / (H / 2) <= 8 / 10), stored after the forward of the tile before
     const int ntiles = (a.B + RT - 1) / RT, nrec_el = RT * R4;
-    float pre[8];
+    float pre[NPRE];
     auto fetch = [&](int tile) {
 #pragma unroll
-        for (int k = 0; k < 8; k++) {
+        for (int k = 0; k < NPRE; k++) {
             const int i = tid + k * (int)blockDim.x;
             pre[k] = 0.f;
             if (tile < ntiles && i < nrec_el) {
@@ -260,11 +271,11 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
     };
     auto store = [&](int buf) {
 #pragma unroll
-        for (int k = 0; k < 8; k++) {
+        for (int k = 0; k < NPRE; k++) {
             const int i = tid + k * (int)blockDim.x;
             if (i < nrec_el) {
                 const int r = i / R4, j = i - r * R4;
-                if (j < P) s_x[(buf * RT + r) * WIDE_MAXP + j] = (pre[k] - s_bn[2 * j]) * s_bn[2 * j + 1];
+                if (j < P) s_x[(buf * RT + r) * PX + j] = (pre[k] - s_bn[2 * j]) * s_bn[2 * j + 1];
                 else if (j - P < ONE_FY) s_fy[(buf * RT + r) * ONE_FY + j - P] = pre[k];
             }
         }
@@ -279,13 +290,13 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
     for (int tile = blockIdx.x; tile < ntiles; tile += gridDim.x, it++) {
         const int buf = it % 3;
         fetch(tile + gridDim.x);
-        const float* xs = s_x + (buf * RT + grp * ONE_R) * WIDE_MAXP;
+        const float* xs = s_x + (buf * RT + grp * ONE_R) * PX;
         switch (a.act) {
-        case ACT_TANH: one_forward_p<ACT_TANH, NOUT>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
-        case ACT_SIGMOID: one_forward_p<ACT_SIGMOID, NOUT>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
-        case ACT_RELU: one_forward_p<ACT_RELU, NOUT>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
-        case ACT_SWISH: one_forward_p<ACT_SWISH, NOUT>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
-        default: one_forward_p<ACT_IDENTITY, NOUT>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
+        case ACT_TANH: one_forward_p<ACT_TANH, NOUT, PX, NO>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
+        case ACT_SIGMOID: one_forward_p<ACT_SIGMOID, NOUT, PX, NO>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
+        case ACT_RELU: one_forward_p<ACT_RELU, NOUT, PX, NO>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
+        case ACT_SWISH: one_forward_p<ACT_SWISH, NOUT, PX, NO>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
+        default: one_forward_p<ACT_IDENTITY, NOUT, PX, NO>(P, xs, w1, b1, wo, A, Gd, s_part[warp], lane); break;
         }
         store((it + 1) % 3);
         __syncthreads();
@@ -386,9 +397,13 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
         if (a.mode != ONE_TRAIN) continue;
         // ---- backward of my units over my group's rows ----
         const float* dzg = s_dz + grp * ONE_R;
-        if (P <= 2) one_backward<2, NOUT>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
-        else if (P <= 4) one_backward<4, NOUT>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
-        else one_backward<8, NOUT>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
+        if constexpr (PX > WIDE_MAXP) {
+            one_backward<PX, NOUT, PX, NO>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
+        } else {
+            if (P <= 2) one_backward<2, NOUT, PX, NO>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
+            else if (P <= 4) one_backward<4, NOUT, PX, NO>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
+            else one_backward<8, NOUT, PX, NO>(xs, dzg, wo, A, Gd, gW1, gb, gWo);
+        }
     }
 
     if (a.mode != ONE_TRAIN) {
@@ -413,7 +428,7 @@ __global__ void __launch_bounds__(ONE_THREADS, 2) k_wide_one(const OneArgs a)
         mine[NOUT * H] = gb.x;
         mine[NOUT * H + 1] = gb.y;
 #pragma unroll
-        for (int p = 0; p < WIDE_MAXP; p++)
+        for (int p = 0; p < PX; p++)
             if (p < P) { mine[(NOUT + 1 + p) * H] = gW1[p].x; mine[(NOUT + 1 + p) * H + 1] = gW1[p].y; }
     }
     // row-thread scalars: dbo, loss sums, phi sums (warp tree, then warps in order)
