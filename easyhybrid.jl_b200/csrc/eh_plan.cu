@@ -11,35 +11,43 @@ namespace rt {
 namespace {
 // Plan for the tensor-core path: one or several Dense chains embedded block-diagonally into one padded chain
 // (eh_wide_kernels.cuh, WideDims).  Fills the parts of the ctx the shared host code reads (record layout, slots, loss,
-// optimiser) and the WideModel handed to WideNet::create.
+// optimiser) and the WideModel handed to WideNet::create.  Chains that differ in depth or activation (2..6 hidden layers)
+// take the per-unit form: a shallower chain carries its last hidden layer up to layer NH on pass-through units (weight 1
+// from the unit below, bias 0, identity activation: exact in bf16), and every hidden unit has its own activation.
 eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
 {
     const int NC = d->n_chains;
     const eh_chain_desc& c0 = d->chains[0];
-    const int NH = c0.n_hidden;
+    int NH = 0;
+    for (int k = 0; k < NC; k++) NH = std::max(NH, d->chains[k].n_hidden);
     int P = 0, NOUT = 0, wl[8] = {0};
+    bool per_unit = false, per_unit_ok = true;
     for (int k = 0; k < NC; k++) {
         const eh_chain_desc& ch = d->chains[k];
-        if (ch.n_hidden != NH || ch.activation != c0.activation || (ch.input_batchnorm != 0) != (c0.input_batchnorm != 0))
-            return fail(c, EH_EUNSUPPORTED, "chains of one model must share depth, activation and input_batchnorm on the tensor-core path");
+        if ((ch.input_batchnorm != 0) != (c0.input_batchnorm != 0))
+            return fail(c, EH_EUNSUPPORTED, "chains of one model must share input_batchnorm on the tensor-core path");
         if (ch.n_in < 1 || ch.n_out < 1) return fail(c, EH_EINVAL, "chain %d: n_in / n_out must be positive", k);
+        per_unit |= ch.n_hidden != NH || ch.activation != c0.activation;
+        per_unit_ok &= ch.activation == EH_ACT_TANH || ch.activation == EH_ACT_SIGMOID || ch.activation == EH_ACT_RELU ||
+                       ch.activation == EH_ACT_IDENTITY;
         P += ch.n_in;
         NOUT += ch.n_out;
-        for (int l = 0; l < ch.n_hidden && l < 8; l++) {
+        for (int l = 0; l < ch.n_hidden && l < 8; l++)
             if (ch.hidden[l] < 1) return fail(c, EH_EINVAL, "chain %d: hidden width must be positive", k);
-            wl[l] += ch.hidden[l];
-        }
+        for (int l = 0; l < NH && l < 8; l++) wl[l] += ch.hidden[std::min(l, ch.n_hidden - 1)];   // (pass-through units too)
     }
     int hmax = 0;
     for (int l = 0; l < NH && l < 8; l++) hmax = std::max(hmax, wl[l]);
-    if (NH > 7 || !eh::wide::WideNet::supported(P, hmax, NH, NOUT, c0.activation, d->process_model))
+    if (NH > 7 || !eh::wide::WideNet::supported(P, hmax, NH, NOUT, c0.activation, d->process_model) ||
+        (per_unit && (NH < 2 || !per_unit_ok)))
         return fail(c, EH_EUNSUPPORTED,
                     "no fused kernel for this model: the register-tile kernels serve 1..3 hidden layers of summed width <= 32 "
-                    "(all activations, <= 8 inputs, <= 2 outputs); the wide path serves 1..4 chains of equal depth, activation "
-                    "and input_batchnorm with <= 12 inputs and <= 4 outputs in total (more than 8 / 2 only with some layer "
-                    "wider than 32; 3..4 outputs: traced process models): one hidden layer of summed width 33..512 (exact fp32, "
-                    "all activations) or 2..6 hidden layers of summed width <= 512 per layer (bf16 tensor cores, tanh / "
-                    "sigmoid / relu) "
+                    "(all activations, <= 8 inputs, <= 2 outputs); the wide path serves 1..4 chains with one input_batchnorm "
+                    "setting and <= 12 inputs and <= 4 outputs in total (more than 8 / 2 only with some layer wider than 32; "
+                    "3..4 outputs: traced process models): one hidden layer of summed width 33..512 (exact fp32, all "
+                    "activations, one activation for all chains) or 2..6 hidden layers of summed width <= 512 per layer, "
+                    "pass-through units of shallower chains included (bf16 tensor cores, tanh / sigmoid / relu; chains may "
+                    "differ in depth and activation) "
                     "(got process_model=%d chains=%d inputs=%d hidden=%d x (<= %d) outputs=%d activation=%d)",
                     d->process_model, NC, P, NH, hmax, NOUT, c0.activation);
     // (one hidden layer: the fused exact-fp32 kernel k_wide_one, images padded to a multiple of 64 units)
@@ -53,7 +61,7 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     wv.T = is_prog ? d->n_targ : ((d->process_model == EH_PM_LINEAR2 || d->process_model == EH_PM_EXPO2) ? 2 : 1);
     wv.R4 = rup4(wv.P + wv.F + wv.T);
     wv.NW = 0; wv.NPART = NSTAT; wv.off_stats = 0; wv.stage_floats = NSTAT; wv.max_warps = 8;
-    wv.name = NH == 1 ? "wide/fp32-one-hidden" : "wide/bf16-tcgen05";
+    wv.name = NH == 1 ? "wide/fp32-one-hidden" : per_unit ? "wide/bf16-tcgen05-per-unit" : "wide/bf16-tcgen05";
     if (wv.T != d->n_targ) return fail(c, EH_EINVAL, "process model yields %d targets, descriptor has %d", wv.T, d->n_targ);
     const Variant* v = &wv;
     c->var = v; c->var2 = nullptr;
@@ -67,10 +75,13 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     c->pm_id = d->process_model;
 
     // flat layout (reference ComponentArray order): chain after chain, per layer W (out x in, column-major) then b; then phi.
-    // Embedding: chain k owns units [uoff[l], uoff[l] + h) of hidden layer l, inputs [ioff, ioff + n_in), outputs [ooff, ..)
+    // Embedding: chain k owns units [uoff[l], uoff[l] + h) of hidden layer l, inputs [ioff, ioff + n_in), outputs [ooff, ..);
+    // a chain of depth dk < NH owns its pass-through units in layers dk + 1 .. NH, and its output layer reads those of NH
     c->h_wmap.assign((size_t)0, 0);
     eh::wide::WideModel& wm = c->wide_model;
     memset(&wm, 0, sizeof wm);
+    wm.per_unit = per_unit ? 1 : 0;
+    memset(wm.uact, EH_ACT_IDENTITY, sizeof wm.uact);
     int off = 0, ioff = 0, ooff = 0, uoff[8] = {0};
     std::vector<int> out_row0((size_t)NC, 0);
     std::vector<std::pair<int, int>> wranges;   // (flat offset, count) of every Dense weight matrix, with its chain in l2_chain
@@ -78,27 +89,39 @@ eh_status build_plan_wide(eh_ctx* c, const eh_model_desc* d, bool is_prog)
     auto push = [&](int kind, int l, int r, int cc) { c->h_wmap.push_back(kind); c->h_wmap.push_back(l); c->h_wmap.push_back(r); c->h_wmap.push_back(cc); };
     for (int k = 0; k < NC; k++) {
         const eh_chain_desc& ch = d->chains[k];
+        const int dk = ch.n_hidden;
         out_row0[k] = ooff;
-        for (int l = 1; l <= NH + 1; l++) {
-            const int hout = l <= NH ? ch.hidden[l - 1] : ch.n_out;
+        for (int l = 1; l <= dk + 1; l++) {
+            const bool outl = l == dk + 1;
+            const int hout = outl ? ch.n_out : ch.hidden[l - 1];
             const int hin = l == 1 ? ch.n_in : ch.hidden[l - 2];
-            const int ro = l <= NH ? uoff[l - 1] : ooff;             // image row origin (output units)
-            const int co = l == 1 ? ioff : uoff[l - 2];              // image column origin (input units)
-            if (l >= 2 && l <= NH) {
+            const int ro = outl ? ooff : uoff[l - 1];                        // image row origin (output units)
+            const int co = l == 1 ? ioff : uoff[outl ? NH - 1 : l - 2];      // image column origin (input units)
+            const int li = outl ? NH + 1 : l;                                // layer of the embedded chain
+            if (!outl && l >= 2) {
                 if (wm.n_blocks >= 32) return fail(c, EH_EUNSUPPORTED, "too many weight blocks");
                 auto& bk = wm.blocks[wm.n_blocks++];
                 bk.l = l; bk.flat_off = off; bk.hout = hout; bk.hin = hin; bk.o_off = ro; bk.i_off = co;
             }
-            const int kind = l == 1 ? eh::wide::WK_W1 : (l <= NH ? eh::wide::WK_WH : eh::wide::WK_WO);
+            const int kind = l == 1 ? eh::wide::WK_W1 : (outl ? eh::wide::WK_WO : eh::wide::WK_WH);
             for (int i = 0; i < hin; i++)
-                for (int o = 0; o < hout; o++) push(kind, l, ro + o, co + i);
+                for (int o = 0; o < hout; o++) push(kind, li, ro + o, co + i);
             wranges.push_back({off, hout * hin});
             l2_chain.push_back(k);
             off += hout * hin;
-            for (int o = 0; o < hout; o++) push(l <= NH ? eh::wide::WK_B : eh::wide::WK_BO, l, ro + o, 0);
+            for (int o = 0; o < hout; o++) push(outl ? eh::wide::WK_BO : eh::wide::WK_B, li, ro + o, 0);
             off += hout;
         }
-        for (int l = 0; l < NH; l++) uoff[l] += ch.hidden[l];
+        for (int l = 1; l <= NH && l <= 6; l++) {
+            const int w = ch.hidden[std::min(l, dk) - 1];
+            memset(&wm.uact[l - 1][uoff[l - 1]], l <= dk ? ch.activation : (int)EH_ACT_IDENTITY, (size_t)w);
+            if (l > dk) {   // pass-through run: unit j of layer l - 1 -> unit j of layer l
+                if (wm.n_pass >= 24) return fail(c, EH_EUNSUPPORTED, "too many pass-through runs");
+                auto& pr = wm.pass[wm.n_pass++];
+                pr.l = l; pr.r0 = uoff[l - 1]; pr.c0 = uoff[l - 2]; pr.n = w;
+            }
+        }
+        for (int l = 0; l < NH; l++) uoff[l] += ch.hidden[std::min(l, dk - 1)];
         ioff += ch.n_in;
         ooff += ch.n_out;
     }
@@ -419,7 +442,8 @@ eh_status build_plan(eh_ctx* c, const eh_model_desc* d)
     // Chains of different depth (hidden sizes differ per parameter, GenericHybridModel.jl:169-189): the embedded chain
     // has the depth of the deepest one; a shallower chain carries its last hidden layer forward through pass-through
     // units (weight 1 from the unit below, no bias, identity activation -- cells fed by no flat entry) up to the common
-    // output layer.  Only the generic variants know pass-through units.
+    // output layer.  The generic variants know pass-through units, and so does the tensor-core path (build_plan_wide) once
+    // some layer is wider than 32 units.
     int Pt = 0, Ot = 0, wsum[8] = {0, 0, 0, 0, 0, 0, 0, 0};
     bool uniform = true, same_depth = true, same_act = true, any_swish = false;
     int NHmax = 0;
@@ -530,10 +554,11 @@ eh_status build_plan(eh_ctx* c, const eh_model_desc* d)
             }
         }
     }
-    if (!v && !same_act)
+    // (chains that differ in activation or depth with some layer wider than 32 units: the tensor-core path's per-unit form)
+    if (!v && !same_act && hmax <= 32)
         return fail(c, EH_EUNSUPPORTED, "chains that differ in activation need run-time compilation (NVRTC; not with EH_JIT=0) on the exact-fp32 "
                                         "generic kernels: <= 3 hidden layers, summed width <= 32 per layer, <= 12 chain inputs, <= 4 chain outputs");
-    if (!v && !same_depth)
+    if (!v && !same_depth && hmax <= 32)
         return fail(c, EH_EUNSUPPORTED, "chains of different depth run on the exact-fp32 generic kernels only: <= 3 hidden layers, "
                                         "summed width <= 32 per layer, <= 12 chain inputs, <= 4 chain outputs");
     if (!v) return build_plan_wide(c, d, is_prog);

@@ -69,26 +69,50 @@ cudaError_t gemm_prepare()
     done = true;
     return cudaSuccess;
 }
+// the per-unit-activation instantiations (chains that differ in depth or activation): set up only for such models
+static cudaError_t gemm_prepare_pu()
+{
+    static bool done = false;
+    if (done) return cudaSuccess;
+    cudaError_t e;
+    if ((e = cudaFuncSetAttribute(k_wide_gemm<GEMM_FWD, WIDE_MAXP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem(GEMM_FWD))) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(k_wide_gemm<GEMM_BWD, WIDE_MAXP, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem(GEMM_BWD))) != cudaSuccess) return e;
+    if ((e = cudaFuncSetAttribute(k_wide_gemm<GEMM_BWD, WIDE_MAXP_X, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, gemm_smem(GEMM_BWD))) != cudaSuccess) return e;
+    for (int cl = 1; cl <= 2; cl++) {
+        const void* fns[3] = {cl == 1 ? (const void*)k_wide_gemm_p<GEMM_FWD, 1, WIDE_MAXP, true> : (const void*)k_wide_gemm_p<GEMM_FWD, 2, WIDE_MAXP, true>,
+                              cl == 1 ? (const void*)k_wide_gemm_p<GEMM_BWD, 1, WIDE_MAXP, true> : (const void*)k_wide_gemm_p<GEMM_BWD, 2, WIDE_MAXP, true>,
+                              cl == 1 ? (const void*)k_wide_gemm_p<GEMM_BWD, 1, WIDE_MAXP_X, true> : (const void*)k_wide_gemm_p<GEMM_BWD, 2, WIDE_MAXP_X, true>};
+        for (const void* f : fns)
+            if ((e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, PG_SMEM)) != cudaSuccess) return e;
+    }
+    done = true;
+    return cudaSuccess;
+}
 
 // out = act(A W^T + bias): A [M x K] bf16, W [N x K] bf16 (K contiguous in both)
 cudaError_t gemm_fwd(const CUtensorMap& tmA, const CUtensorMap& tmW, int M, int N, int K, const float* bias, int act,
-                     __nv_bfloat16* out, cudaStream_t st)
+                     __nv_bfloat16* out, cudaStream_t st, const uint8_t* uact)
 {
     GemmArgs g{};
-    g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.bias = bias; g.out16 = out;
-    k_wide_gemm<GEMM_FWD><<<dim3(M / BM, N / gemm_bn(GEMM_FWD), 1), GEMM_THREADS, gemm_smem(GEMM_FWD), st>>>(tmA, tmW, g);
+    g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.bias = bias; g.out16 = out; g.uact = uact;
+    const dim3 grid(M / BM, N / gemm_bn(GEMM_FWD), 1);
+    if (uact) k_wide_gemm<GEMM_FWD, WIDE_MAXP, true><<<grid, GEMM_THREADS, gemm_smem(GEMM_FWD), st>>>(tmA, tmW, g);
+    else k_wide_gemm<GEMM_FWD><<<grid, GEMM_THREADS, gemm_smem(GEMM_FWD), st>>>(tmA, tmW, g);
     return cudaGetLastError();
 }
 // out = (D Wt^T) .* act'(aux): D [M x K] bf16, Wt [N x K] bf16, aux [M x N] bf16
 cudaError_t gemm_bwd(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int N, int K, const __nv_bfloat16* aux, int act,
                      __nv_bfloat16* out, cudaStream_t st, float* colsum, const float* xb, const float* bscal, int R4, int P1,
-                     int use_bn)
+                     int use_bn, const uint8_t* uact)
 {
     GemmArgs g{};
     g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.aux = aux; g.out16 = out;
-    g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn;
+    g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn; g.uact = uact;
     const dim3 grid(M / BM, N / gemm_bn(GEMM_BWD), 1);
-    if (P1 > WIDE_MAXP) k_wide_gemm<GEMM_BWD, WIDE_MAXP_X><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
+    if (uact) {
+        if (P1 > WIDE_MAXP) k_wide_gemm<GEMM_BWD, WIDE_MAXP_X, true><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
+        else k_wide_gemm<GEMM_BWD, WIDE_MAXP, true><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
+    } else if (P1 > WIDE_MAXP) k_wide_gemm<GEMM_BWD, WIDE_MAXP_X><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
     else k_wide_gemm<GEMM_BWD><<<grid, GEMM_THREADS, gemm_smem(GEMM_BWD), st>>>(tmD, tmWt, g);
     return cudaGetLastError();
 }
@@ -98,7 +122,7 @@ cudaError_t gemm_bwd(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int
 // single CTAs: the kernels are bound by shared-memory bandwidth -- TMA writes plus MMA operand reads -- not by L2 reads).
 static bool pg_cluster() { static const bool on = getenv("EH_WIDE_CLUSTER") != nullptr; return on; }
 int pg_box_rows() { return pg_cluster() ? PG_BN / 2 : PG_BN; }
-template <int MODE, int PX = WIDE_MAXP>
+template <int MODE, int PX = WIDE_MAXP, bool PU = false>
 static cudaError_t launch_gemm_p(const CUtensorMap& tmA, const CUtensorMap& tmB, const GemmArgs& g, cudaStream_t st)
 {
     static int nsm = 0, max_clusters = -1;
@@ -122,20 +146,20 @@ static cudaError_t launch_gemm_p(const CUtensorMap& tmA, const CUtensorMap& tmB,
         if (max_clusters < 0) {
             cfg.gridDim = dim3((unsigned)(nsm & ~1));
             int mc = 0;
-            if (cudaOccupancyMaxActiveClusters(&mc, k_wide_gemm_p<MODE, 2, PX>, &cfg) != cudaSuccess || mc < 1) { cudaGetLastError(); mc = 0; }
+            if (cudaOccupancyMaxActiveClusters(&mc, k_wide_gemm_p<MODE, 2, PX, PU>, &cfg) != cudaSuccess || mc < 1) { cudaGetLastError(); mc = 0; }
             max_clusters = mc;
         }
         if (max_clusters > 0) {
             const int units = (mt / 2) * nn;
             const int ncl = std::min(std::min(max_clusters, nsm / 2), units);
             cfg.gridDim = dim3((unsigned)(2 * ncl));
-            return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 2, PX>, tmA, tmB, g);
+            return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 2, PX, PU>, tmA, tmB, g);
         }
         cfg.attrs = nullptr;
         cfg.numAttrs = 0;
     }
     cfg.gridDim = dim3((unsigned)std::min(mt * nn, nsm));
-    return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 1, PX>, tmA, tmB, g);
+    return cudaLaunchKernelEx(&cfg, k_wide_gemm_p<MODE, 1, PX, PU>, tmA, tmB, g);
 }
 int persistent_grid(int M, int N)
 {
@@ -149,19 +173,24 @@ int persistent_grid(int M, int N)
     return tiles < nsm ? tiles : nsm;
 }
 cudaError_t gemm_fwd_p(const CUtensorMap& tmA, const CUtensorMap& tmW, int M, int N, int K, const float* bias, int act,
-                       __nv_bfloat16* out, cudaStream_t st)
+                       __nv_bfloat16* out, cudaStream_t st, const uint8_t* uact = nullptr)
 {
     GemmArgs g{};
-    g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.bias = bias; g.out16 = out;
+    g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.bias = bias; g.out16 = out; g.uact = uact;
+    if (uact) return launch_gemm_p<GEMM_FWD, WIDE_MAXP, true>(tmA, tmW, g, st);
     return launch_gemm_p<GEMM_FWD>(tmA, tmW, g, st);
 }
 cudaError_t gemm_bwd_p(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int N, int K, const __nv_bfloat16* aux, int act,
                        __nv_bfloat16* out, cudaStream_t st, float* colsum, const float* xb, const float* bscal, int R4, int P1,
-                       int use_bn)
+                       int use_bn, const uint8_t* uact = nullptr)
 {
     GemmArgs g{};
     g.M = M; g.N = N; g.K = K; g.ksplits = 1; g.act = act; g.aux = aux; g.out16 = out;
-    g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn;
+    g.colsum = colsum; g.xb = xb; g.bscal = bscal; g.R4 = R4; g.P1 = P1; g.use_bn = use_bn; g.uact = uact;
+    if (uact) {
+        if (P1 > WIDE_MAXP) return launch_gemm_p<GEMM_BWD, WIDE_MAXP_X, true>(tmD, tmWt, g, st);
+        return launch_gemm_p<GEMM_BWD, WIDE_MAXP, true>(tmD, tmWt, g, st);
+    }
     if (P1 > WIDE_MAXP) return launch_gemm_p<GEMM_BWD, WIDE_MAXP_X>(tmD, tmWt, g, st);
     return launch_gemm_p<GEMM_BWD>(tmD, tmWt, g, st);
 }
@@ -183,22 +212,26 @@ cudaError_t gemm_wgrad(const CUtensorMap& tmD, const CUtensorMap& tmA, int M, in
 namespace {
 
 typedef void (*HeadKernel)(const HeadArgs);
-struct HeadEntry { int pm, nout, scale, hch, aff; HeadKernel fn; };
-#define EH_HEAD(PMF, NOUT, SCALE, HCH, AFF) {PMF::ID, NOUT, SCALE, HCH, AFF, k_wide_head<HeadCfg<PMF, NOUT, (SCALE != 0), (AFF != 0)>, HCH>},
-#define EH_HEAD_PMA(PMF, AFF) EH_HEAD(PMF, 1, 0, 1, AFF) EH_HEAD(PMF, 1, 1, 1, AFF) EH_HEAD(PMF, 2, 0, 1, AFF) EH_HEAD(PMF, 2, 1, 1, AFF) \
-                              EH_HEAD(PMF, 1, 0, 2, AFF) EH_HEAD(PMF, 1, 1, 2, AFF) EH_HEAD(PMF, 2, 0, 2, AFF) EH_HEAD(PMF, 2, 1, 2, AFF)
-#define EH_HEAD_PM(PMF) EH_HEAD_PMA(PMF, 0) EH_HEAD_PMA(PMF, 1)
+struct HeadEntry { int pm, nout, scale, hch, aff, pu; HeadKernel fn; };
+#define EH_HEAD(PMF, NOUT, SCALE, HCH, AFF, PU) {PMF::ID, NOUT, SCALE, HCH, AFF, PU, k_wide_head<HeadCfg<PMF, NOUT, (SCALE != 0), (AFF != 0), (PU != 0)>, HCH>},
+#define EH_HEAD_PMA(PMF, AFF, PU) EH_HEAD(PMF, 1, 0, 1, AFF, PU) EH_HEAD(PMF, 1, 1, 1, AFF, PU) EH_HEAD(PMF, 2, 0, 1, AFF, PU) EH_HEAD(PMF, 2, 1, 1, AFF, PU) \
+                                  EH_HEAD(PMF, 1, 0, 2, AFF, PU) EH_HEAD(PMF, 1, 1, 2, AFF, PU) EH_HEAD(PMF, 2, 0, 2, AFF, PU) EH_HEAD(PMF, 2, 1, 2, AFF, PU)
+#define EH_HEAD_PM(PMF, PU) EH_HEAD_PMA(PMF, 0, PU) EH_HEAD_PMA(PMF, 1, PU)
 // three and four outputs: traced process models only (the built-in forms have two parameters)
-#define EH_HEAD_PMA34(PMF, AFF) EH_HEAD(PMF, 3, 0, 1, AFF) EH_HEAD(PMF, 3, 1, 1, AFF) EH_HEAD(PMF, 4, 0, 1, AFF) EH_HEAD(PMF, 4, 1, 1, AFF) \
-                                EH_HEAD(PMF, 3, 0, 2, AFF) EH_HEAD(PMF, 3, 1, 2, AFF) EH_HEAD(PMF, 4, 0, 2, AFF) EH_HEAD(PMF, 4, 1, 2, AFF)
-const HeadEntry g_heads[] = {EH_HEAD_PM(PmRbQ10) EH_HEAD_PM(PmExpo) EH_HEAD_PM(PmLinear) EH_HEAD_PM(PmLinear2) EH_HEAD_PM(PmExpo2)
-                             EH_HEAD_PM(PmProgram) EH_HEAD_PMA34(PmProgram, 0) EH_HEAD_PMA34(PmProgram, 1)};
+#define EH_HEAD_PMA34(PMF, AFF, PU) EH_HEAD(PMF, 3, 0, 1, AFF, PU) EH_HEAD(PMF, 3, 1, 1, AFF, PU) EH_HEAD(PMF, 4, 0, 1, AFF, PU) EH_HEAD(PMF, 4, 1, 1, AFF, PU) \
+                                    EH_HEAD(PMF, 3, 0, 2, AFF, PU) EH_HEAD(PMF, 3, 1, 2, AFF, PU) EH_HEAD(PMF, 4, 0, 2, AFF, PU) EH_HEAD(PMF, 4, 1, 2, AFF, PU)
+#define EH_HEAD_ALL(PU) EH_HEAD_PM(PmRbQ10, PU) EH_HEAD_PM(PmExpo, PU) EH_HEAD_PM(PmLinear, PU) EH_HEAD_PM(PmLinear2, PU) EH_HEAD_PM(PmExpo2, PU) \
+                        EH_HEAD_PM(PmProgram, PU) EH_HEAD_PMA34(PmProgram, 0, PU) EH_HEAD_PMA34(PmProgram, 1, PU)
+// pu = 1: the training heads of models whose chains differ in depth or activation (act' per unit)
+const HeadEntry g_heads[] = {EH_HEAD_ALL(0) EH_HEAD_ALL(1)};
 
-// aff: the training head of a model with LOSS_AFFINE targets (the statistics and evaluation modes take aff = 0)
-HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false)
+// aff: the training head of a model with LOSS_AFFINE targets (the statistics and evaluation modes take aff = 0); pu: the
+// training head of a per-unit-activation model (the statistics and evaluation modes need no act' and take pu = 0)
+HeadKernel find_head(int pm, int nout, int scale, int hch, bool aff = false, bool pu = false)
 {
     for (const HeadEntry& e : g_heads)
-        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0) && e.hch == hch && e.aff == (aff ? 1 : 0)) return e.fn;
+        if (e.pm == pm && e.nout == nout && e.scale == (scale ? 1 : 0) && e.hch == hch && e.aff == (aff ? 1 : 0) && e.pu == (pu ? 1 : 0))
+            return e.fn;
     return nullptr;
 }
 
@@ -283,9 +316,13 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
         w->one_max_ = std::max(1, per_sm) * m.nsm;
     } else if ((e = gemm_prepare()) != cudaSuccess) {
         return bail("gemm_prepare", e);
+    } else if (m.per_unit && (e = gemm_prepare_pu()) != cudaSuccess) {
+        return bail("gemm_prepare", e);
     }
-    for (int aff = 0; aff <= (w->affine_ ? 1 : 0) && m.NH >= 2; aff++) {
-        HeadKernel hk = find_head(m.pm, m.NOUT, m.scale, m.H / 256, aff != 0);
+    // (a per-unit model's training head is the pu form, the last round; statistics and evaluation take the plain one)
+    for (int aff = 0; aff <= (w->affine_ ? 1 : 0) + (m.per_unit ? 1 : 0) && m.NH >= 2; aff++) {
+        const bool pu = m.per_unit && aff == (w->affine_ ? 2 : 1);
+        HeadKernel hk = pu ? find_head(m.pm, m.NOUT, m.scale, m.H / 256, w->affine_, true) : find_head(m.pm, m.NOUT, m.scale, m.H / 256, aff != 0);
         if (!hk) { snprintf(err, errlen, "wide path: no head kernel for this process model / shape"); delete w; return nullptr; }
         const int head_smem = (8 * (m.NOUT + 1) + m.NOUT) * m.H * (int)sizeof(float);   // warps' scratch / row rings + the output-layer weights
         e = cudaFuncSetAttribute((const void*)hk, cudaFuncAttributeMaxDynamicSharedMemorySize, head_smem);
@@ -308,6 +345,30 @@ WideNet* WideNet::create(const WideModel& m, char* err, size_t errlen)
             delete w;
             return nullptr;
         }
+    }
+    if (m.per_unit && m.NH >= 2) {
+        // pass-through units: weight 1 from the unit below (bias 0, identity activation), exact in bf16.  No flat entry
+        // maps to these cells, so k_wide_update never overwrites them
+        std::vector<__nv_bfloat16> img;
+        for (int l = 2; l <= m.NH; l++) {
+            bool any = false;
+            for (int i = 0; i < m.n_pass; i++) any |= m.pass[i].l == l;
+            if (!any) continue;
+            for (int dir = 0; dir < 2; dir++) {   // Wf [out][in], Wb [in][out]
+                img.assign(HH, __float2bfloat16(0.f));
+                for (int i = 0; i < m.n_pass; i++)
+                    for (int j = 0; m.pass[i].l == l && j < m.pass[i].n; j++) {
+                        const size_t r = (size_t)(m.pass[i].r0 + j), c = (size_t)(m.pass[i].c0 + j);
+                        img[dir == 0 ? r * m.H + c : c * m.H + r] = __float2bfloat16(1.f);
+                    }
+                if ((e = cudaMemcpy(dir == 0 ? w->Wf_[l - 1] : w->Wb_[l - 1], img.data(), HH * 2, cudaMemcpyHostToDevice)) != cudaSuccess)
+                    return bail("cudaMemcpy", e);
+            }
+        }
+        if ((e = cudaMalloc(&w->uact_, (size_t)m.NH * m.H)) != cudaSuccess) return bail("cudaMalloc", e);
+        for (int l = 1; l <= m.NH; l++)
+            if ((e = cudaMemcpy(w->uact_ + (size_t)(l - 1) * m.H, m.uact[l - 1], (size_t)m.H, cudaMemcpyHostToDevice)) != cudaSuccess)
+                return bail("cudaMemcpy", e);
     }
     if (m.NH == 1) {
         const size_t cs = (size_t)w->one_max_ * (1 + m.P) * m.H * 4;
@@ -376,7 +437,7 @@ WideNet::~WideNet()
         if (colsum_[i]) cudaFree(colsum_[i]);
     }
     void* ps[] = {xb_, D_[0], D_[1], partial_, head_partial_, stats_, skip_, evalpart_, l2part_, ticket_, d_prog_, W1img_, WOimg_, BOimg_,
-                  d_map_, d_small_};
+                  d_map_, d_small_, uact_};
     for (void* p : ps)
         if (p) cudaFree(p);
 }
@@ -445,15 +506,26 @@ cudaError_t WideNet::forward(const float* rec, const int* idx, long long rec_bas
     const int rows_per_cta = (256 / (H / 8)) * FIRST_ROWS;
     {
         const unsigned g1 = (unsigned)((B + rows_per_cta - 1) / rows_per_cta);
-        if (d.P <= 2) k_wide_first<2><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
-        else if (d.P <= 4) k_wide_first<4><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
-        else if (d.P <= WIDE_MAXP) k_wide_first<8><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
-        else k_wide_first<WIDE_MAXP_X><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0]);
+        const uint8_t* ua = uact_;   // (per-unit models: the chains' activations of layer 1)
+#define EH_FIRST(PM_, PU_) k_wide_first<PM_, PU_><<<g1, 256, 0, st>>>(xb_, W1img_, Bp_[0], bscal, m_.use_bn, d, B, m_.act, A_[0], ua)
+        if (!ua) {
+            if (d.P <= 2) EH_FIRST(2, false);
+            else if (d.P <= 4) EH_FIRST(4, false);
+            else if (d.P <= WIDE_MAXP) EH_FIRST(8, false);
+            else EH_FIRST(WIDE_MAXP_X, false);
+        } else {
+            if (d.P <= 2) EH_FIRST(2, true);
+            else if (d.P <= 4) EH_FIRST(4, true);
+            else if (d.P <= WIDE_MAXP) EH_FIRST(8, true);
+            else EH_FIRST(WIDE_MAXP_X, true);
+        }
+#undef EH_FIRST
     }
     WN(cudaGetLastError());
     for (int l = 2; l <= m_.NH; l++) {
-        if (persist_) WN(gemm_fwd_p(tmA_k_[l - 2], tmWf_[l - 1], B, H, H, Bp_[l - 1], m_.act, A_[l - 1], st));
-        else WN(gemm_fwd(tmA_k_[l - 2], tmWf_[l - 1], B, H, H, Bp_[l - 1], m_.act, A_[l - 1], st));
+        const uint8_t* ua = uact_ ? uact_ + (size_t)(l - 1) * H : nullptr;
+        if (persist_) WN(gemm_fwd_p(tmA_k_[l - 2], tmWf_[l - 1], B, H, H, Bp_[l - 1], m_.act, A_[l - 1], st, ua));
+        else WN(gemm_fwd(tmA_k_[l - 2], tmWf_[l - 1], B, H, H, Bp_[l - 1], m_.act, A_[l - 1], st, ua));
     }
     return cudaSuccess;
 }
@@ -486,9 +558,10 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
     WN(ensure(B));
     WN(forward(rec, idx, rec_base, 1ll << 62, B, Bvalid, bscal, pblock, st));
     const WideDims d = dims_of(m_);
-    HeadKernel hk = find_head(m_.pm, m_.NOUT, m_.scale, H / 256, affine_);
+    HeadKernel hk = find_head(m_.pm, m_.NOUT, m_.scale, H / 256, affine_, uact_ != nullptr);
     HeadArgs ha{};
     ha.A = A_[NH - 1]; ha.xb = xb_; ha.pblock = pblock; ha.WOimg = WOimg_; ha.BOimg = BOimg_; ha.bscal = bscal; ha.D = D_[NH & 1];
+    ha.uact = uact_ ? uact_ + (size_t)(NH - 1) * H : nullptr;
     ha.partial = head_partial_;
     ha.d = d; ha.B = B; ha.Bvalid = Bvalid; ha.act = m_.act; ha.train = 1;
     ha.prog = reinterpret_cast<const PmProgData*>(d_prog_); ha.nf = m_.F; ha.nt = m_.T;
@@ -537,12 +610,13 @@ cudaError_t WideNet::step(const float* rec, const int* idx, long long rec_base, 
         if (fork) { WN(cudaEventRecord(ev_wred_, side_)); pending = true; }
         // backward data; its epilogue also leaves the 32-row column sums of D_{l-1} (bias gradient of layer l-1 and,
         // for layer 1, the x-weighted sums = its weight gradient)
+        const uint8_t* ua = uact_ ? uact_ + (size_t)(l - 2) * H : nullptr;   // act' of layer l - 1
         if (persist_)
             WN(gemm_bwd_p(tmD_k_[cur], tmWb_[l - 1], B, H, H, A_[l - 2], m_.act, D_[nxt], st, colsum_[l - 2], xb_, bscal, m_.R4,
-                          (l - 1 == 1) ? m_.P : 0, m_.use_bn));
+                          (l - 1 == 1) ? m_.P : 0, m_.use_bn, ua));
         else
             WN(gemm_bwd(tmD_k_[cur], tmWb_[l - 1], B, H, H, A_[l - 2], m_.act, D_[nxt], st, colsum_[l - 2], xb_, bscal, m_.R4,
-                        (l - 1 == 1) ? m_.P : 0, m_.use_bn));
+                        (l - 1 == 1) ? m_.P : 0, m_.use_bn, ua));
     }
     if (pending) WN(cudaStreamWaitEvent(st, ev_wred_, 0));   // the flat gradient is complete from here on
     return finish_step(n_head_, n_slab_, bscal, pblock, m, v, ost, grad, grad_final, loss_out, apply, st, dp);

@@ -10,11 +10,12 @@ namespace wide {
 
 bool make_map_bf16(CUtensorMap* map, const void* ptr, uint64_t inner, uint64_t rows, uint64_t pitch_elems, uint32_t box_rows);
 cudaError_t gemm_prepare();
+// uact: NULL, or [N] activation codes per output column (chains that differ in depth or activation)
 cudaError_t gemm_fwd(const CUtensorMap& tmA, const CUtensorMap& tmW, int M, int N, int K, const float* bias, int act,
-                     __nv_bfloat16* out, cudaStream_t st);
+                     __nv_bfloat16* out, cudaStream_t st, const uint8_t* uact = nullptr);
 cudaError_t gemm_bwd(const CUtensorMap& tmD, const CUtensorMap& tmWt, int M, int N, int K, const __nv_bfloat16* aux, int act,
                      __nv_bfloat16* out, cudaStream_t st, float* colsum, const float* xb, const float* bscal, int R4, int P1,
-                     int use_bn);
+                     int use_bn, const uint8_t* uact = nullptr);
 cudaError_t gemm_wgrad(const CUtensorMap& tmD, const CUtensorMap& tmA, int M, int N, int Kall, int ksplits, float* partial,
                        cudaStream_t st);
 
@@ -53,6 +54,13 @@ struct WideModel {          // filled by eh_lib's planner from the model descrip
     short prog_op[48], prog_a[48], prog_b[48];
     float prog_imm[48];
     int prog_out[4];
+    // chains that differ in depth or activation (2..6 hidden layers): the activation of every embedded hidden unit
+    // (ACT_IDENTITY for pass-through and padding units) and the pass-through runs, W_l[r0 + j][c0 + j] = 1 for j < n, that
+    // carry a shallower chain's last hidden layer up to layer NH.  per_unit = 0: `act` for every unit, no pass-through
+    int per_unit;
+    unsigned char uact[6][512];
+    int n_pass;
+    struct { int l, r0, c0, n; } pass[24];
 };
 
 // the wide-chain training step: owns activations / deltas / bf16 weight images / partial buffers
@@ -126,6 +134,7 @@ private:
     int* d_small_ = nullptr;   // flat indices assembled by k_wide_gradfin
     int n_small_ = 0;
     void* d_prog_ = nullptr;   // PmProgData on the device
+    uint8_t* uact_ = nullptr;  // per_unit: [NH][H] activation codes of the hidden units
     float* partial_ = nullptr;
     // the split-K reductions (latency-bound, a few CTAs) run on a side stream next to the backward-data GEMM of their layer
     cudaStream_t side_ = nullptr;

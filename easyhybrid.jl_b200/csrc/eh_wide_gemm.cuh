@@ -61,6 +61,9 @@ struct GemmArgs {
     const float* xb;         // [M x R4] compact batch records (first P1 entries = chain inputs)
     const float* bscal;      // input BatchNorm scalars (mu, rstd per input) when use_bn
     int R4, P1, use_bn;
+    // PU instantiations (chains that differ in depth or activation): ACT_* per column of the output (FWD) / of aux
+    // (BWD) instead of `act`, [N] bytes
+    const uint8_t* uact;
 };
 
 // ---- thin PTX wrappers ---------------------------------------------------------------------------
@@ -177,6 +180,14 @@ __device__ __forceinline__ float dact1(int act, float a)
     if (act == ACT_RELU) return a > 0.f ? 1.f : 0.f;
     return 1.f;
 }
+// per-unit activations: the codes of 32 consecutive columns (16-byte aligned) as eight words, the same in every lane
+__device__ __forceinline__ void load_acts32(const uint8_t* uact, uint32_t (&w)[8])
+{
+    const uint4 a = __ldg(reinterpret_cast<const uint4*>(uact)), b = __ldg(reinterpret_cast<const uint4*>(uact) + 1);
+    w[0] = a.x; w[1] = a.y; w[2] = a.z; w[3] = a.w; w[4] = b.x; w[5] = b.y; w[6] = b.z; w[7] = b.w;
+}
+template <int N>
+__device__ __forceinline__ int act_at(const uint32_t (&w)[N], int j) { return (int)((w[j >> 2] >> (8 * (j & 3))) & 0xffu); }
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
 {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
@@ -186,8 +197,9 @@ __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi)
 // grid: (M / BM, N / BN, ksplits).  FWD / BWD: tmA = [M x K] K-major (box 64 x 128), tmB = [N x K] K-major
 // (box 64 x 128).  WGRAD: tmA = deltas [Kall x M], tmB = activations [Kall x N], both MN-major (box 64 x 64).
 // PX: chain inputs the backward-data epilogue's input-weighted column sums hold (WIDE_MAXP, or WIDE_MAXP_X in the
-// instantiation that serves the layer-1 call of models with more than WIDE_MAXP inputs)
-template <int MODE, int PX = WIDE_MAXP>
+// instantiation that serves the layer-1 call of models with more than WIDE_MAXP inputs).  PU: activation per column
+// (g.uact), a separate instantiation so that the others keep their code
+template <int MODE, int PX = WIDE_MAXP, bool PU = false>
 __global__ void __launch_bounds__(GEMM_THREADS, MODE == GEMM_WGRAD ? 1 : 2)
 k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g)
 {
@@ -313,13 +325,19 @@ k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                                          __uint_as_float(r[4 * j + 3]));
             } else {
                 uint32_t o[16];
+                uint32_t uw[PU ? 8 : 1];
+                if constexpr (PU) load_acts32(g.uact + n0 + c, uw);
+                auto act_of = [&](int j) {   // column c + j
+                    if constexpr (PU) return act_at(uw, j);
+                    else return g.act;
+                };
                 if (MODE == GEMM_FWD) {
                     const float4* b4 = reinterpret_cast<const float4*>(s_bias + c);
 #pragma unroll
                     for (int j = 0; j < 8; j++) {
                         const float4 b = b4[j];
-                        o[2 * j] = pack_bf16(act1(g.act, __uint_as_float(r[4 * j]) + b.x), act1(g.act, __uint_as_float(r[4 * j + 1]) + b.y));
-                        o[2 * j + 1] = pack_bf16(act1(g.act, __uint_as_float(r[4 * j + 2]) + b.z), act1(g.act, __uint_as_float(r[4 * j + 3]) + b.w));
+                        o[2 * j] = pack_bf16(act1(act_of(4 * j), __uint_as_float(r[4 * j]) + b.x), act1(act_of(4 * j + 1), __uint_as_float(r[4 * j + 1]) + b.y));
+                        o[2 * j + 1] = pack_bf16(act1(act_of(4 * j + 2), __uint_as_float(r[4 * j + 2]) + b.z), act1(act_of(4 * j + 3), __uint_as_float(r[4 * j + 3]) + b.w));
                     }
                 } else {
 #pragma unroll
@@ -330,8 +348,8 @@ k_wide_gemm(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUt
                         for (int e = 0; e < 4; e++) {
                             const __nv_bfloat162 ab = *reinterpret_cast<const __nv_bfloat162*>(&aw[e]);
                             const float2 af = __bfloat1622float2(ab);
-                            o[4 * j + e] = pack_bf16(__uint_as_float(r[8 * j + 2 * e]) * dact1(g.act, af.x),
-                                                     __uint_as_float(r[8 * j + 2 * e + 1]) * dact1(g.act, af.y));
+                            o[4 * j + e] = pack_bf16(__uint_as_float(r[8 * j + 2 * e]) * dact1(act_of(8 * j + 2 * e), af.x),
+                                                     __uint_as_float(r[8 * j + 2 * e + 1]) * dact1(act_of(8 * j + 2 * e + 1), af.y));
                         }
                     }
                 }
@@ -458,8 +476,9 @@ __device__ __forceinline__ void cluster_sync_all()
 // weight tile of a stage (128 of the 256 rows) and multicasts it into both, so a tile costs 256 KB of L2 reads instead of
 // 384 KB -- the kernel runs at the L2 throughput limit (about 12 TB/s), not at the tensor pipe's.  A stage is reusable
 // when BOTH CTAs' MMAs have read it (the commits arrive on both empty barriers).  tmB: box of BN rows for CL = 1, BN / 2 for CL = 2.
-// PX: as for k_wide_gemm (the staged strip of a warp, 32 x PG_OPITCH bytes, holds the (1 + PX) x PG_CW parked sums)
-template <int MODE, int CL, int PX = WIDE_MAXP>
+// PX: as for k_wide_gemm (the staged strip of a warp, 32 x PG_OPITCH bytes, holds the (1 + PX) x PG_CW parked sums).
+// PU: as for k_wide_gemm
+template <int MODE, int CL, int PX = WIDE_MAXP, bool PU = false>
 __global__ void __launch_bounds__(PG_THREADS, 1)
 k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB, const GemmArgs g)
 {
@@ -606,6 +625,12 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
             for (int cc = 0; cc < NCC; cc++) {
                 const int c = cc * 32;
                 uint32_t r[32];
+                uint32_t uw[PU ? 8 : 1];
+                if constexpr (PU) load_acts32(g.uact + ncol0 + c, uw);
+                auto act_of = [&](int j) {   // column ncol0 + c + j
+                    if constexpr (PU) return act_at(uw, j);
+                    else return g.act;
+                };
                 tc_ld_32x32(tmem_base + ((uint32_t)(q * 32) << 16) + (uint32_t)(ab * BN + h * CW + c), r);
                 uint32_t o[16];
                 if (MODE == GEMM_FWD) {
@@ -613,8 +638,8 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
                     for (int j = 0; j < 8; j++) {
                         const float4 b = b4[j];
-                        o[2 * j] = pack_bf16(act1(g.act, __uint_as_float(r[4 * j]) + b.x), act1(g.act, __uint_as_float(r[4 * j + 1]) + b.y));
-                        o[2 * j + 1] = pack_bf16(act1(g.act, __uint_as_float(r[4 * j + 2]) + b.z), act1(g.act, __uint_as_float(r[4 * j + 3]) + b.w));
+                        o[2 * j] = pack_bf16(act1(act_of(4 * j), __uint_as_float(r[4 * j]) + b.x), act1(act_of(4 * j + 1), __uint_as_float(r[4 * j + 1]) + b.y));
+                        o[2 * j + 1] = pack_bf16(act1(act_of(4 * j + 2), __uint_as_float(r[4 * j + 2]) + b.z), act1(act_of(4 * j + 3), __uint_as_float(r[4 * j + 3]) + b.w));
                     }
                 } else {
                     // this thread's own row of the activation strip; the result goes back to the same bytes
@@ -625,8 +650,8 @@ k_wide_gemm_p(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ C
 #pragma unroll
                         for (int e = 0; e < 4; e++) {
                             const float2 af = __bfloat1622float2(*reinterpret_cast<const __nv_bfloat162*>(&aw[e]));
-                            o[4 * j + e] = pack_bf16(__uint_as_float(r[8 * j + 2 * e]) * dact1(g.act, af.x),
-                                                     __uint_as_float(r[8 * j + 2 * e + 1]) * dact1(g.act, af.y));
+                            o[4 * j + e] = pack_bf16(__uint_as_float(r[8 * j + 2 * e]) * dact1(act_of(8 * j + 2 * e), af.x),
+                                                     __uint_as_float(r[8 * j + 2 * e + 1]) * dact1(act_of(8 * j + 2 * e + 1), af.y));
                         }
                     }
                 }

@@ -79,16 +79,26 @@ __device__ __forceinline__ uint32_t pack2(float lo, float hi) { return pack_bf16
 constexpr int FIRST_ROWS = 16;
 // PMAX: compile-time bound on the chain inputs (2 / 4 / 8 / 12) -- the weights a thread keeps in registers.  Rows go four at
 // a time with their inputs loaded first: the kernel is a stream of 16-byte stores (H bf16 per row) and must not wait for
-// one L2 round trip per row.
-template <int PMAX>
+// one L2 round trip per row.  PU: activation per unit (uact [H] bytes) instead of `act`.
+template <int PMAX, bool PU = false>
 __global__ void __launch_bounds__(256) k_wide_first(const float* __restrict__ xb, const float* __restrict__ W1img,
                                                     const float* __restrict__ b1img, const float* __restrict__ bscal, int use_bn,
-                                                    WideDims d, int B, int act, __nv_bfloat16* __restrict__ A1)
+                                                    WideDims d, int B, int act, __nv_bfloat16* __restrict__ A1,
+                                                    const uint8_t* __restrict__ uact)
 {
     const int per_row = d.H / 8;                       // threads across the width
     const int groups = 256 / per_row;                  // row groups per CTA
     const int o0 = (threadIdx.x % per_row) * 8;
     const int r0 = (blockIdx.x * groups + threadIdx.x / per_row) * FIRST_ROWS;
+    uint32_t uw[2] = {0u, 0u};
+    if constexpr (PU) {
+        const uint2 u = __ldg(reinterpret_cast<const uint2*>(uact + o0));
+        uw[0] = u.x; uw[1] = u.y;
+    }
+    auto act_of = [&](int j) {   // unit o0 + j
+        if constexpr (PU) return act_at(uw, j);
+        else return act;
+    };
     float bias[8], w[PMAX][8], mu[PMAX], rs[PMAX];
 #pragma unroll
     for (int j = 0; j < 8; j++) bias[j] = __ldg(b1img + o0 + j);
@@ -116,22 +126,23 @@ __global__ void __launch_bounds__(256) k_wide_first(const float* __restrict__ xb
 #pragma unroll
                 for (int j = 0; j < 8; j++) z[j] = fmaf(x[i][p], w[p][j], z[j]);
             uint4 o;
-            o.x = pack2(act_bf16(act, z[0]), act_bf16(act, z[1]));
-            o.y = pack2(act_bf16(act, z[2]), act_bf16(act, z[3]));
-            o.z = pack2(act_bf16(act, z[4]), act_bf16(act, z[5]));
-            o.w = pack2(act_bf16(act, z[6]), act_bf16(act, z[7]));
+            o.x = pack2(act_bf16(act_of(0), z[0]), act_bf16(act_of(1), z[1]));
+            o.y = pack2(act_bf16(act_of(2), z[2]), act_bf16(act_of(3), z[3]));
+            o.z = pack2(act_bf16(act_of(4), z[4]), act_bf16(act_of(5), z[5]));
+            o.w = pack2(act_bf16(act_of(6), z[6]), act_bf16(act_of(7), z[7]));
             if (b0 + i < B) *reinterpret_cast<uint4*>(A1 + (size_t)(b0 + i) * d.H + o0) = o;
         }
     }
 }
 
 // the pieces of StepCfg that resolve_params / the process-model functors look at.  AFF: the training mode knows LOSS_AFFINE
-// seeds (a separate instantiation: the kernel runs at its register limit, and the extra case must not cost the others)
-template <class PM_, int NOUT_, bool SCALE_, bool AFF_ = false>
+// seeds (a separate instantiation: the kernel runs at its register limit, and the extra case must not cost the others).
+// PU: the training mode takes act' per unit of A_NH (HeadArgs::uact), for chains that differ in depth or activation
+template <class PM_, int NOUT_, bool SCALE_, bool AFF_ = false, bool PU_ = false>
 struct HeadCfg {
     using PM = PM_;
     static constexpr int NOUT = NOUT_, NPS = PM_::NPS, T = PM_::NT, F = PM_::NF;
-    static constexpr bool SCALE = SCALE_, AFF = AFF_;
+    static constexpr bool SCALE = SCALE_, AFF = AFF_, PU = PU_;
 };
 
 struct HeadArgs {
@@ -156,6 +167,7 @@ struct HeadArgs {
     float pmc[4];
     const PmProgData* prog;    // device copy of the traced program (PmProgram heads), else NULL
     int nf, nt;                // real forcing / target counts (PmProgram heads; the built-in forms know theirs)
+    const uint8_t* uact;       // HeadCfg::PU: [H] ACT_* per unit of A_NH (ACT_IDENTITY: pass-through and padding units)
 };
 
 // ---- output layer + physics + loss seeds + backward into D_NH; one warp per sample row, 8 warps per CTA ----
@@ -367,6 +379,15 @@ __global__ void __launch_bounds__(256, head_ctas_per_sm(HC::NOUT)) k_wide_head(c
 #pragma unroll
         for (int c = 0; c < HCH; c++) {
             float dv[8], av[8], sacc[8];
+            uint32_t uw[2] = {0u, 0u};
+            if constexpr (HC::PU) {
+                const uint2 u = __ldg(reinterpret_cast<const uint2*>(a.uact + (c * 32 + lane) * 8));
+                uw[0] = u.x; uw[1] = u.y;
+            }
+            auto act_of = [&](int e) {   // feature (c * 32 + lane) * 8 + e
+                if constexpr (HC::PU) return act_at(uw, e);
+                else return a.act;
+            };
             load_av(c, av);
 #pragma unroll
             for (int e = 0; e < 8; e++) sacc[e] = 0.f;
@@ -383,7 +404,7 @@ __global__ void __launch_bounds__(256, head_ctas_per_sm(HC::NOUT)) k_wide_head(c
 #pragma unroll
             for (int e = 0; e < 8; e++) {
                 // round first: db must be the column sum of the very deltas the weight-gradient GEMM reads
-                dv[e] = __bfloat162float(__float2bfloat16_rn(sacc[e] * dact_out(a.act, av[e])));
+                dv[e] = __bfloat162float(__float2bfloat16_rn(sacc[e] * dact_out(act_of(e), av[e])));
                 gDb[c][e] += dv[e];
             }
             uint4 o4;

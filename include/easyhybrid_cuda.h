@@ -333,8 +333,11 @@ eh_status eh_set_profiling(eh_ctx* ctx, int32_t on);
 /* which compiled kernel family serves this ctx (static string, never NULL), e.g.
  * "ffma2/PmRbQ10/P2/NH2/H16/O1/ACT_TANH/scale=true" (exact-fp32 register-tile kernels, specialised form),
  * "ffma2/PmProgram/..." (same kernels, process model interpreted per sample), "wide/bf16-tcgen05" or, for one hidden layer
- * of 33..512 units, "wide/fp32-one-hidden".  The two wide families take 1..4 chains of equal depth, activation and
- * input_batchnorm with <= 12 chain inputs and <= 4 chain outputs in total (3..4 outputs: traced process models).
+ * of 33..512 units, "wide/fp32-one-hidden".  The two wide families take 1..4 chains of one input_batchnorm setting with
+ * <= 12 chain inputs and <= 4 chain outputs in total (3..4 outputs: traced process models); chains of one hidden layer share
+ * their activation.  Chains that differ in depth or activation (tanh / sigmoid / relu, 2..6 hidden layers) train on the
+ * tensor cores as "wide/bf16-tcgen05-per-unit": shallower chains ride on pass-through units, every unit has its own
+ * activation, and the summed width per layer (pass-through units included) is <= 512.
  * The reference has no counterpart; callers use it to report / assert the path a model took.          */
 const char* eh_kernel_variant(const eh_ctx* ctx);
 /* Plans `desc` as eh_create would and compiles its traced process model with NVRTC (EH_FLAG_JIT implied) WITHOUT touching a
